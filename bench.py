@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference's CPU path
+    python bench.py --steps K --dump-outputs DIR                    # + the last timed step's outputs as DIR/*.npy
 
 A *step* is one pass of the hot path over one batch of synthetic Zipf(1.05) indices
 (26 tables x B samples): probe -> EvLFU promote -> miss fetch from the host-pinned backing
@@ -44,7 +45,7 @@ def log(*a):
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps of the value line (the e2e and roofline legs time as many)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="samples per step (default 2048)")
@@ -79,7 +80,31 @@ def parse_args():
                     help="table shape: kaggle (configs[1-3]) or terabyte (configs[4]: dim 64, cardinalities capped at 40 M); N = 1 with "
                          "terabyte needs --table-slice (one rank's tables fit one host, all 48 GB of them do not)")
     ap.add_argument("--table-slice", default="", help="N = 1 only: serve tables a:b of the shape, e.g. 0:4 = what rank 0 of an 8-GPU run owns")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="N = 1 only: after the timed steps, write what the last timed step returned (rows [B, T, dim], hit codes "
+                         "[B, T]) as DIR/rows.npy and DIR/hit.npy in float32; above 64 MB a seeded sample of the samples, whose "
+                         "indices go to DIR/sample.npy.  The same arguments give the same inputs, so two builds compare file by file")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.op or a.gpus > 1):
+        ap.error("--dump-outputs applies to the N = 1 line of our CUDA path")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, rows: np.ndarray, hit: np.ndarray) -> None:
+    """rows [B, T, dim] fp32, hit [B, T] uint8 of one step -> path/*.npy (float32), at most DUMP_BYTES in all."""
+    os.makedirs(path, exist_ok=True)
+    B = rows.shape[0]
+    per_sample = rows[0].size * 4 + hit[0].size * 4 + 8
+    arrays = {"rows": rows, "hit": hit.astype(np.float32)}
+    if B * per_sample > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_sample, replace=False))
+        arrays = {"rows": rows[keep], "hit": arrays["hit"][keep], "sample": keep.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a))
+    log("outputs of the last timed step written to %s: %s" % (path, {k: list(v.shape) for k, v in arrays.items()}))
 
 
 class ClockSampler:
@@ -465,9 +490,9 @@ def main_ours(args):
 
     store.phase_times()                           # clears the debug accumulators
     # ---- value: indices resident in HBM ------------------------------------------------------
-    # Three regions of EXACTLY K steps each, W warm-up steps before the first; the line reports the median region (a
-    # 20-step region is 0.6 ms: box-to-box and run-to-run spread of anything that touches PCIe is +-10 %) and lists all.
-    # Every step announces the next index batch (evs_prefetch), as a serving loop with its requests queued would.
+    # EXACTLY K timed steps, W warm-up steps before them, in up to three back-to-back regions of whole calls (listed in
+    # value_regions_ms, so that a region that stands out is visible); the line reports all K steps over the summed region
+    # time.  Every step announces the next index batch (evs_prefetch), as a serving loop with its requests queued would.
     base = warm
     for k in range(W):
         store.lookup(idx_dev[base + k], out=out, hit=hit)
@@ -484,10 +509,13 @@ def main_ours(args):
     import ctypes as C
     out_ptrs = (C.c_void_p * GROUP)(*([out.data_ptr()] * GROUP))
     hit_ptrs = (C.c_void_p * GROUP)(*([hit.data_ptr()] * GROUP))
-    for rep in range(3):
+    n_calls = -(-K // GROUP)
+    region_steps = [GROUP * (n_calls // 3 + (r < n_calls % 3)) for r in range(min(3, n_calls))]
+    region_steps[-1] -= sum(region_steps) - K              # the last call may hold fewer than GROUP batches
+    for Kr in region_steps:
         l0 = store.launch_count()
-        calls = [(k, min(GROUP, K - k), (C.c_void_p * GROUP)(*[idx_dev[base + k + j].data_ptr() for j in range(GROUP)]))
-                 for k in range(0, K, GROUP)]
+        calls = [(k, min(GROUP, Kr - k), (C.c_void_p * GROUP)(*[idx_dev[base + k + j].data_ptr() for j in range(GROUP)]))
+                 for k in range(0, Kr, GROUP)]
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for k, n, ips in calls:
@@ -497,14 +525,16 @@ def main_ours(args):
         e1.record()
         torch.cuda.synchronize()
         regions.append(e0.elapsed_time(e1))
-        launches = store.launch_count() - l0
-        base += K
-    ms_dev = sorted(regions)[1]
+        launches += store.launch_count() - l0
+        base += Kr
+    # every batch of a call writes the same buffers: they hold the last timed step's result until the legs below reuse them
+    last_step = (out.cpu().numpy(), hit.cpu().numpy()) if args.dump_outputs else None
+    ms_dev = sum(regions)
     base -= W + K                                 # the sections below advance by W + K
     phases = store.phase_times()
     log("device phases of the last timed batch (us):", phases)
     st = store.stats(reset=True)
-    KK = 3 * K
+    KK = K
     log("per step: misses %.0f evictions %.0f flushed %.0f inserts %.0f" % (st["misses"] / KK, st["evictions"][0] / KK,
         st["flushed"][0] / KK, st["inserts"][0] / KK))
     hit_rate = (st["hits"][0] + st["hits"][1] + st["c3_hits"]) / max(1, st["lookups"])
@@ -766,12 +796,14 @@ def main_ours(args):
         "cache": {"fill": fill, "hbm_bytes": footprint, "budget_bytes": cache_rows * dim * prec // 8,
                   "note": "hbm_bytes = index (load factor <= 1/3) + slot-indexed slab + bucket rings + look-ahead staging; budget_bytes "
                           "= cache rows x row bytes, the reference's TOTAL_SIZE accounting (cache_manager.cpp:16)"},
-        "value_regions_ms": regions, "look_ahead": use_pf, "batches_per_call": GROUP, "configs4": configs4, "other_configs": other, "ops": ops,
+        "value_regions_ms": regions, "value_region_steps": region_steps, "look_ahead": use_pf, "batches_per_call": GROUP, "configs4": configs4, "other_configs": other, "ops": ops,
         "e2e": {"value": e2e_value, "unit": "lookups/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                 "ms_per_step": 1e3 * e2e_s / K, "api": "evs_submit_host/evs_wait_host (4 batches in flight)",
                 "sync_call_value": lookups / e2e_sync_s, "sync_call_ms_per_step": 1e3 * e2e_sync_s / K},
         "gpu_launches": int(launches), "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu,
     }
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, *last_step)
     print(json.dumps(line), flush=True)
     if store is not None:
         store.close()

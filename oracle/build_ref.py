@@ -2,7 +2,7 @@
 """Compile the reference's own C++ cache (mixed_precs_caching/) into oracle/_ref/*.so.
 
 TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).  The sources are read where they lie
-under /root/reference; nothing of them is copied into this repository.  Because the
+in the checkout named by EVSTORE_REFERENCE; nothing of them is copied into this repository.  Because the
 reference's configuration is compile-time text (cache_manager.cpp:13-20 #defines,
 EV_DIMENSION in every header, hard-coded /mnt/extra/... data roots in evlfu_*.hpp:58-64 and
 aprx_embedding.hpp:39), each variant is built from a *patched stream* of those files placed
@@ -12,7 +12,8 @@ reference's own compile line (cache_manager.cpp:10):
     g++ -shared -o libcachemanager.so -fPIC -O3 evlfu_4.cpp evlfu_8.cpp evlfu_16.cpp
         evlfu_32.cpp [aprx_embedding.cpp] cache_manager.cpp -pthread
 
-Outputs go to oracle/_ref/ only (git-ignored, travels to the GPU box with gpurun).
+Outputs go to oracle/_ref/ only (git-ignored).  Without a reference checkout only our own
+helpers are built (libref_drive.so, libstdset_shim.so).
 """
 import os
 import re
@@ -23,9 +24,9 @@ import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
-from oracle.ref_variants import FIXTURE_ROOT, VARIANTS, lib_name  # noqa: E402
+from oracle.ref_variants import FIXTURE_ROOT, REFERENCE, VARIANTS, lib_name  # noqa: E402
 
-REF_SRC = "/root/reference/mixed_precs_caching"
+REF_SRC = os.path.join(REFERENCE, "mixed_precs_caching") if REFERENCE else ""
 OUT = os.path.join(HERE, "_ref")
 SOURCES = ["evlfu_4.cpp", "evlfu_8.cpp", "evlfu_16.cpp", "evlfu_32.cpp", "aprx_embedding.cpp", "cache_manager.cpp"]
 HEADERS = ["evlfu_4.hpp", "evlfu_8.hpp", "evlfu_16.hpp", "evlfu_32.hpp", "aprx_embedding.hpp", "cache_manager.hpp"]
@@ -94,8 +95,8 @@ def build_shim(force: bool = False) -> str:
 def main(argv):
     build_driver(force="--force" in argv)
     build_shim(force="--force" in argv)
-    if not os.path.isdir(REF_SRC):
-        print("oracle/build_ref.py: /root/reference is absent; using prebuilt oracle/_ref/*.so")
+    if not REF_SRC or not os.path.isdir(REF_SRC):
+        print("oracle/build_ref.py: no reference checkout (EVSTORE_REFERENCE); built the oracle's own helpers only")
         return 0
     names = [a for a in argv if not a.startswith("-")] or list(VARIANTS)
     for n in names:

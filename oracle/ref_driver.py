@@ -66,7 +66,7 @@ class RefCache:
         self.variant, self.dim, self.n_tables = variant, v["dim"], 26
         path = os.path.join(REF_DIR, lib_name(variant))
         if not os.path.exists(path):
-            raise RuntimeError(f"{path} missing: run oracle/build_ref.py where /root/reference exists")
+            raise RuntimeError(f"{path} missing: run oracle/build_ref.py with EVSTORE_REFERENCE set")
         if fresh_copy:
             import shutil
             import tempfile

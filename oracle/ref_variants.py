@@ -3,10 +3,15 @@
 The reference fixes its cache configuration, its embedding dimension and its data root at
 compile time (mixed_precs_caching/cache_manager.cpp:13-20, cache_manager.hpp:30-31,
 evlfu_32.hpp:61 ...), so every configuration we time or compare against is a separate .so.
-``oracle/build_ref.py`` compiles each entry below from the sources where they lie under
-/root/reference into ``oracle/_ref/lib<name>.so``; the fixture files the library opens at
-dlopen time are written by the caller (bench.py / tests) under FIXTURE_ROOT/<fixture>/.
+``oracle/build_ref.py`` compiles each entry below from the sources of a checkout of the
+original project (the directory named by the EVSTORE_REFERENCE environment variable) into
+``oracle/_ref/lib<name>.so``; the fixture files the library opens at dlopen time are written by
+the caller (bench.py / tests) under FIXTURE_ROOT/<fixture>/.
 """
+import os
+
+# checkout of the original project (its cache_algo/ and mixed_precs_caching/), or "" when there is none
+REFERENCE = os.environ.get("EVSTORE_REFERENCE", "")
 
 # the compiled-in data root; /dev/shm keeps the CPU baseline off the disk (BASELINE.md section 3)
 FIXTURE_ROOT = "/dev/shm/evstore_b200_ref/"

@@ -116,7 +116,7 @@ def _load_shim():
     if _shim is None:
         p = os.path.join(HERE, "_ref", "libstdset_shim.so")
         if not os.path.exists(p):
-            raise RuntimeError(f"{p} missing: run oracle/build_ref.py")
+            raise RuntimeError(f"{p} missing: run build() (python __graft_entry__.py), which compiles it")
         lib = C.CDLL(p)
         lib.uset_new.restype = C.c_void_p
         lib.uset_free.argtypes = [C.c_void_p]

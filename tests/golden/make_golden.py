@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generate golden vectors by running the UNMODIFIED reference code.
 
-Run in the build container only (needs /root/reference); the outputs
+Needs a checkout of the original project, named by EVSTORE_REFERENCE; the outputs
 (``tests/golden/*.npz``) are committed, this script is how they were made.
 
-  python tests/golden/make_golden.py
+  EVSTORE_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 1. ``evlfu_c1_*.npz``   -- /root/reference/cache_algo/EvLFU_C1.py driven one request
    at a time on synthetic Zipf traces with a stub ``storage_manager`` whose rows
@@ -18,7 +18,8 @@ Run in the build container only (needs /root/reference); the outputs
 6. ``lfu_*.npz``        -- /root/reference/cache_algo/LFU.py: per request hit vector and the set of evicted keys,
    plus the final frequency lists and least_freq.
 5. ``dlrm_forward.npz`` -- the reference's DLRM_Net (BASELINE configs[0] architecture, small tables) run on the CPU:
-   weights, one input batch, interaction output and click probabilities.
+   one input batch, interaction output, click probabilities and the SHA-256 of every weight / table array
+   (tests/helpers.py load_dlrm_golden redraws them from the seed).
 4. ``formats/``         -- files written by the reference's own writers: the big-endian alt-key binary
    (script/convert_altkeys_to_binary.py) from ``altkeys.txt``, and ``training_config.txt`` (evstore_utils.py).
 """
@@ -28,7 +29,7 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ.get("EVSTORE_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 T = 26
 DIM = 36                     # the reference's hard-coded EV_DIMENSION
@@ -333,6 +334,8 @@ def golden_dlrm():
     (13 dense, 26 tables, dim 16, bot 13-512-256-64-16, top 367-512-256-1, dot interaction), small random
     tables, one batch of 128 through sequential_forward on the CPU.  Saved: every weight, the inputs, the
     click probabilities -- the end-to-end known answer for bottom MLP -> lookup -> interaction -> top MLP."""
+    import hashlib
+
     import torch
     sys.path.insert(0, REF)
     sys.path.insert(0, os.path.join(REF, "script"))
@@ -355,14 +358,16 @@ def golden_dlrm():
         x = net.apply_mlp(X, net.bot_l)
         ly = net.apply_emb(lS_o, lS_i, net.emb_l, net.v_W_l)
         R = net.interact_features(x, ly)
-    out = dict(rows=np.array(rows), X=X.numpy(), lS_i=lS_i.numpy(), Z=Z.numpy(), R=R.numpy())
-    for k, e in enumerate(net.emb_l):
-        out[f"emb_{k}"] = e.weight.detach().numpy()
+    out = dict(rows=np.array(rows), X=X.numpy(), lS_i=lS_i.numpy(), Z=Z.numpy(), R=R.numpy(), seed=np.array(777))
+    # the weights and tables are ~2 MB of random floats: store their digests; tests/helpers.load_dlrm_golden redraws them
+    arrays = {f"emb_{k}": e.weight for k, e in enumerate(net.emb_l)}
     for name, mlp in (("bot", net.bot_l), ("top", net.top_l)):
         lin = [l for l in mlp if isinstance(l, torch.nn.Linear)]
         for i, l in enumerate(lin):
-            out[f"{name}_w{i}"] = l.weight.detach().numpy()
-            out[f"{name}_b{i}"] = l.bias.detach().numpy()
+            arrays[f"{name}_w{i}"], arrays[f"{name}_b{i}"] = l.weight, l.bias
+    for k, a in arrays.items():
+        digest = hashlib.sha256(np.ascontiguousarray(a.detach().numpy()).tobytes()).digest()
+        out["sha256_" + k] = np.frombuffer(digest, dtype=np.uint8)
     np.savez_compressed(os.path.join(HERE, "dlrm_forward.npz"), **out)
     print("dlrm_forward: Z", Z.shape, float(Z.min()), float(Z.max()), "R", R.shape)
 

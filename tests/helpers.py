@@ -157,6 +157,30 @@ def run_tier_parity(rows, dim, layers, main, sec, total, B_list, n_batches, prop
     return tot
 
 
+def load_dlrm_golden(golden_dir):
+    """tests/golden/dlrm_forward.npz with the weights and tables of the model it was computed with.  The file holds the
+    inputs, the reference's outputs and the SHA-256 of every weight / table array.  The arrays themselves are redrawn
+    here in the order DLRM_Net.__init__ draws them from np.random seeded with `seed` (create_emb: uniform(+-sqrt(1/n))
+    per table; create_mlp for the bottom, then the top MLP: normal(0, sqrt(2/(m+n))) weights, normal(0, sqrt(1/m))
+    biases) and must hash to the stored digests."""
+    import hashlib
+    import os
+    with np.load(os.path.join(golden_dir, "dlrm_forward.npz")) as z:
+        g = {k: z[k] for k in z.files}
+    rng = np.random.RandomState(int(g["seed"]))
+    m_spa = g["R"].shape[1] - 27 * 26 // 2
+    for k, n in enumerate(int(x) for x in g["rows"]):
+        g[f"emb_{k}"] = rng.uniform(low=-np.sqrt(1 / n), high=np.sqrt(1 / n), size=(n, m_spa)).astype(np.float32)
+    for name, ln in (("bot", [g["X"].shape[1], 512, 256, 64, m_spa]), ("top", [g["R"].shape[1], 512, 256, 1])):
+        for i in range(len(ln) - 1):
+            n, m = ln[i], ln[i + 1]
+            g[f"{name}_w{i}"] = rng.normal(0.0, np.sqrt(2 / (m + n)), size=(m, n)).astype(np.float32)
+            g[f"{name}_b{i}"] = rng.normal(0.0, np.sqrt(1 / m), size=m).astype(np.float32)
+    for k in [k for k in g if k.startswith("sha256_")]:
+        assert hashlib.sha256(g[k[7:]].tobytes()).digest() == g[k].tobytes(), f"{k[7:]} differs from the reference's array"
+    return g
+
+
 def dlrm_forward_cpu(g, tables):
     """sequential_forward of the reference's DLRM_Net (dlrm_s_pytorch.py:588-613) restated with plain torch on the
     CPU over the weights of tests/golden/dlrm_forward.npz and the given embedding tables.  Returns (Z [B,1], R [B,367])."""

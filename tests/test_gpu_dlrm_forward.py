@@ -1,22 +1,19 @@
 """BASELINE configs[0] end to end: the reference's own DLRM_Net (Kaggle architecture, small random tables) was
-run on the CPU by tests/golden/make_golden.py; its weights, one input batch, the interaction output and the
-click probabilities are in tests/golden/dlrm_forward.npz.  ``dlrm_ops.DLRMInference.sequential_forward``
+run on the CPU by tests/golden/make_golden.py; one input batch, the interaction output, the click probabilities
+and digests of its weights are in tests/golden/dlrm_forward.npz (helpers.load_dlrm_golden redraws the weights).  ``dlrm_ops.DLRMInference.sequential_forward``
 (bottom MLP on cuBLAS next to the cached lookup, our interaction kernel, top MLP) must reproduce them:
 fp32 rows from the cache are exact copies, so only GEMM summation order differs -- tolerance 2e-6 absolute on
 the probabilities (they lie in 0.29..0.37), 1e-4 / 1e-5 (atol / rtol) on the 367 interaction features."""
-import os
-
 import numpy as np
 import pytest
 
-from helpers import pkg
+from helpers import load_dlrm_golden, pkg
 
 pytestmark = pytest.mark.gpu
 
 
 def _golden(golden_dir):
-    with np.load(os.path.join(golden_dir, "dlrm_forward.npz")) as z:
-        return {k: z[k] for k in z.files}
+    return load_dlrm_golden(golden_dir)
 
 
 @pytest.mark.parametrize("use_cache,policy", [(True, "evlfu"), (True, "lru"), (False, "evlfu")])

@@ -152,9 +152,8 @@ def test_dlrm_forward_golden_describes_the_reference_model(golden_dir):
     """The fixture is self-consistent: recomputing sequential_forward (dlrm_s_pytorch.py:588-613) from the saved
     weights with plain torch on the CPU gives the saved interaction features and probabilities; and the stated
     tolerances of the quantised tiers (tests/test_gpu_dlrm_forward.py) hold for the reference's own codecs."""
-    from helpers import dlrm_forward_cpu
-    with np.load(os.path.join(golden_dir, "dlrm_forward.npz")) as z:
-        g = {k: z[k] for k in z.files}
+    from helpers import dlrm_forward_cpu, load_dlrm_golden
+    g = load_dlrm_golden(golden_dir)
     tables = [g[f"emb_{k}"] for k in range(26)]
     Z, R = dlrm_forward_cpu(g, tables)
     assert np.allclose(R, g["R"], rtol=1e-5, atol=1e-6)

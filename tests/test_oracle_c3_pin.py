@@ -67,7 +67,7 @@ def _compare(out, trace, dec, alt, v):
 @pytest.mark.parametrize("seed,alpha,min_c3", [(5, 1.05, 300), (6, 0.8, 100), (7, 1.3, 100)])
 def test_three_layer_sequential_equals_compiled_reference_driven_slowly(seed, alpha, min_c3):
     if not (ref_driver.available(VARIANT) and tiers.shim_available()):
-        pytest.skip("oracle/_ref not built (run oracle/build_ref.py where /root/reference exists)")
+        pytest.skip("needs the original project's compiled cache (set EVSTORE_REFERENCE to its checkout, run build())")
     p = pkg()
     v = VARIANTS[VARIANT]
     tables = p.workload.make_tables(SMALL_ROWS, DIM)

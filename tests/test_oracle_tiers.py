@@ -1,7 +1,8 @@
 """The multi-layer oracles (oracle/tiers.py) against the reference itself.
 
-The reference's two-layer path exists only in C++; oracle/build_ref.py compiles it from
-/root/reference into oracle/_ref/lib<variant>.so.  ``SeqTiers(order="stdset", flush="cpp")``
+The reference's two-layer path exists only in C++; oracle/build_ref.py (run by build()) compiles it
+from the checkout of the original project named by EVSTORE_REFERENCE into oracle/_ref/lib<variant>.so;
+without one these pins skip.  ``SeqTiers(order="stdset", flush="cpp")``
 must reproduce it request by request: every returned row has to be the dequantised row of the
 tier the restatement says answered (fp32 / 16 / 8 / 4-bit rows of one key differ, so the floats
 identify the tier), over thousands of requests with evictions, promotions and the C1-full
@@ -43,7 +44,7 @@ def _trace(n, seed, alpha=1.05):
 
 def _run_pin(variant, fixture_tables, n, seed, alpha=1.05, fresh=False):
     if not (ref_driver.available(variant) and tiers.shim_available()):
-        pytest.skip("oracle/_ref not built (run oracle/build_ref.py where /root/reference exists)")
+        pytest.skip("needs the original project's compiled cache (set EVSTORE_REFERENCE to its checkout, run build())")
     _tables, raw, dec = fixture_tables
     v = VARIANTS[variant]
     ref_driver.write_fixture(variant, {prec: raw[prec] for prec in PRECS})
