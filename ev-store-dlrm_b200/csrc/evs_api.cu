@@ -626,6 +626,10 @@ int evs_create(const evs_config *cfg, evs_handle *out) {
         set_error("evs_create: bad n_tables / dim / max_batch / rows / n_layers");
         return EVS_ERR_INVALID;
     }
+    if (static_cast<unsigned long long>(cfg->max_batch) * cfg->n_tables > kMaxProtPositions) {
+        set_error("evs_create: max_batch * n_tables must not exceed 2^27 positions");
+        return EVS_ERR_INVALID;
+    }
     evs_handle h = new evs_handle_s();
     h->cfg = *cfg;
     if (h->cfg.n_tables_total <= 0) h->cfg.n_tables_total = cfg->n_tables;

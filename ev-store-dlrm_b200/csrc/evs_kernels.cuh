@@ -945,7 +945,7 @@ __device__ void evict_tier(const TierDev &tier, const Params &p) {
     // evict down to capacity, lowest bucket first, FIFO inside a bucket; the highest ranked
     // new key is never the victim (the reference evicts before it inserts)
     unsigned prot_slot = kNoSlot;
-    if (n_new > 0) prot_slot = __ldcg(p.pos_slot + static_cast<unsigned>(prot & 0xFFFFFFFFull)) & ~kClaimedBit;
+    if (n_new > 0) prot_slot = evs::prot_slot(prot);
     const unsigned need = size > tier.cap ? size - tier.cap : 0u;
     unsigned ev = 0;
     if (need > 0) ev = pop_range(tier, S, 0, top, need, prot_slot, tier.evicted, 0);

@@ -53,6 +53,16 @@ struct __align__(16) Slot {
     unsigned long long meta;
 };
 
+// What a tier's k_evict CTA 0 derives from the counters (its plan), left for whichever CTA closes the batch.
+struct EvictOut {
+    unsigned long long head[kMaxBuckets];      // ring heads before the victims
+    unsigned long long tail[kMaxBuckets];      // ring tails after this batch's appends
+    unsigned long long total_v;                // records of the buckets that give up victims
+    unsigned int count[kMaxBuckets];           // entries per bucket once the victims are out
+    unsigned int take_mask;                    // buckets that give up victims
+    unsigned int size, need, top_left, any_perfect, flush, appended, pad;
+};
+
 struct TierCtl {
     unsigned long long head[kMaxBuckets];
     unsigned long long tail[kMaxBuckets];
@@ -60,7 +70,7 @@ struct TierCtl {
     unsigned long long scan_end[kMaxBuckets];    // k_evict: end of the scanned part of the ring
     unsigned int count[kMaxBuckets];       // live entries per bucket
     unsigned int ticket;                   // k_evict: next eviction chunk
-    unsigned int done_ctas;                // k_evict: CTAs of this tier that finished
+    unsigned int done_ctas;                // k_evict, flush path: CTAs of this tier that have their plan
     unsigned int stop;                     // k_evict: the victims are complete, take no more chunks
     unsigned int n_taken;                  // k_evict: victims evicted by this batch
     unsigned int n_perfect;                // n_perfect_item_C1 (evlfu_32.hpp:51)
@@ -68,13 +78,14 @@ struct TierCtl {
     // per batch (reset by the evict kernel)
     unsigned int n_new;
     unsigned int any_perfect;
-    unsigned long long prot;               // max over new keys of (bucket+1) << 32 | position
+    unsigned long long prot;               // max over new keys of pack_prot(bucket+1, position, slot)
     unsigned int n_evicted_last;
     unsigned int n_flushed_last;
     unsigned int error;
     unsigned int pad;
     // cumulative
     unsigned long long stat_inserts, stat_evictions, stat_flushed;
+    EvictOut out;                          // k_evict: the plan of the batch in flight
 };
 
 struct TierDev {
@@ -208,7 +219,7 @@ struct Params {
     unsigned int *hist;                    // [kSeqs][n_chunks_max]: per-CTA append counts (prefixes after k_scan)
     unsigned int *tot;                     // [kSeqs] batch totals of the same (k_serve adds, k_evict clears)
     unsigned int stage_stride;             // max row_stride of the tiers (shared-memory staging of unaligned rows)
-    unsigned int *done;                    // k_evict: tiers finished (C3 needs both tiers' victims)
+    unsigned int *done;                    // k_evict: CTAs arrived (every eviction CTA, the last fetch CTA); the last closes the batch
     unsigned int *miss_list;               // [N] position | tier << 31 of every miss of the batch in flight
     unsigned int *miss_ctl;                // [0] entries in miss_list, [1] fetch CTAs finished
     int evict_ctas;                        // CTAs per tier of the eviction roles of k_evict
@@ -229,6 +240,15 @@ __host__ __device__ inline unsigned long long pack_meta(int bucket, unsigned lon
 }
 __host__ __device__ inline int meta_bucket(unsigned long long m) { return static_cast<int>(m >> 56) - 1; }
 __host__ __device__ inline unsigned long long meta_pos(unsigned long long m) { return m & 0x00FFFFFFFFFFFFFFull; }
+
+// TierCtl::prot: the batch's newest key (highest (bucket, position) among its claims) together with the slot it claimed, so
+// that the eviction plan has the protected slot without a dependent load.  6 + 27 + 31 bits: positions < 2^27 (evs_create).
+constexpr unsigned long long kMaxProtPositions = 1ull << 27;
+__host__ __device__ inline unsigned long long pack_prot(unsigned bucket1, unsigned pos, unsigned slot) {
+    return (static_cast<unsigned long long>(bucket1) << 58) | (static_cast<unsigned long long>(pos) << 31) | (slot & 0x7FFFFFFFu);
+}
+__host__ __device__ inline int prot_bucket(unsigned long long prot) { return static_cast<int>(prot >> 58) - 1; }
+__host__ __device__ inline unsigned prot_slot(unsigned long long prot) { return static_cast<unsigned>(prot) & 0x7FFFFFFFu; }
 
 __host__ __device__ inline unsigned long long make_key(int table, long long row) {
     return (static_cast<unsigned long long>(table) << kKeyShift) | static_cast<unsigned long long>(row);

@@ -13,7 +13,8 @@
 //              chunks of kEvictWindow records, a CTA's first chunk is its block index, further ones go by ticket, and a chunk
 //              learns how many victims precede it by a decoupled look-back over its predecessors' counts.  A batch that
 //              triggers the flush rule (rare) takes the single-CTA path of evs_kernels.cuh.  Miss-fetch role
-//              (p.fetch_ctas CTAs): fetch_list_body (evs_kernels.cuh).  The last role to finish inserts the victims into
+//              (p.fetch_ctas CTAs): fetch_list_body (evs_kernels.cuh).  Every eviction CTA and the last fetch CTA arrive on
+//              one counter; the last to arrive (close_batch) writes every tier's counters back, inserts the victims into
 //              C3, mirrors the ring occupancy to the host and -- sharded -- exchanges the "rows delivered" words.
 #pragma once
 #include "evs_c3.cuh"
@@ -183,7 +184,7 @@ __global__ void __launch_bounds__(kLookupThreads, COOP ? 3 : (NG == 1 ? 5 : 4)) 
         slot = claim_slot(p.tier[tr], make_key(p.tid[tbl], r), claimed);
         p.pos_slot[pos] = slot | (claimed ? kClaimedBit : 0u);
         if (claimed) atomicAdd(&s_new[tr], 1u);
-        atomicMax(&s_prot[tr], (static_cast<unsigned long long>(f & 0x3Fu) << 32) | static_cast<unsigned>(pos));
+        atomicMax(&s_prot[tr], pack_prot(f & 0x3Fu, static_cast<unsigned>(pos), slot));
     } else if (f) {
         slot = p.pos_slot[pos];
     }
@@ -406,12 +407,137 @@ __device__ __forceinline__ unsigned lookback_excl_wide(unsigned long long *lb, u
     return excl;
 }
 
+// The CTA that arrives last closes the batch.  Its chain is one round of independent loads (every tier's published plan,
+// the chunks' results, the phase stamps), then stores only:
+//   warp t < n_tiers   lane = bucket: write tier t's counters back, reset its per-batch scratch, and keep the longest ring
+//                      window in a register for the host's mirror;
+//   warp kPhaseWarp    lane = phase-accounting word (p.dbg).
+// Then C3, the sharded completion words, the ring mirror (a store into mapped host memory that no fence waits for) and
+// the running phase sums.
+constexpr int kPhaseWarp = kMaxTiers;
+static_assert(kEvictThreads >= (kPhaseWarp + 1) * 32, "close_batch needs a warp per tier plus one");
+__device__ __forceinline__ void close_batch(const Params &p) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned nev = static_cast<unsigned>(p.evict_ctas);
+    unsigned long long used = 0ull;          // warp t < n_tiers: max over tier t's buckets of tail - head
+    unsigned long long d = 0ull, t5 = 0ull;  // warp kPhaseWarp: p.dbg[lane], the closing CTA's start
+    const unsigned seq = p.args->seq;
+    const int world = p.args->sh.world;
+    if (warp < p.n_tiers) {
+        const int t = warp, b = lane;
+        const TierDev &tier = p.tier[t];
+        TierCtl *ctl = tier.ctl;
+        volatile TierCtl *c = ctl;
+        const volatile EvictOut &o = c->out;
+        const bool in = b < tier.n_buckets;
+        const unsigned long long oh = o.head[b], ot = o.tail[b], kept = c->kept[b], se = c->scan_end[b];
+        const unsigned ocnt = o.count[b];
+        const unsigned mask = o.take_mask, size = o.size, need = o.need, top_left = o.top_left, any_perfect = o.any_perfect,
+                       flush = o.flush, appended = o.appended;
+        const unsigned long long total_v = o.total_v;
+        const unsigned taken = c->n_taken, ticket = c->ticket;
+        if (!flush) {
+            unsigned long long head = oh;
+            if ((mask >> b) & 1u) head = (kept != ~0ull) ? kept : (se > oh ? se : oh);
+            if (ocnt == 0) head = ot;
+            if (in) {
+                if (ot - head > tier.ring_cap) c->error = 4u;
+                c->head[b] = head;
+                c->tail[b] = ot;
+                c->count[b] = ocnt;
+                used = ot - head;
+            }
+            if (lane == 0) {
+                if (any_perfect) c->n_perfect = top_left;       // EvLFU_C1.py:163-165
+                atomicAdd(&ctl->stat_evictions, static_cast<unsigned long long>(taken));
+                c->n_evicted_last = taken;
+                c->n_flushed_last = 0;
+                c->full_at_start = (size - taken >= tier.cap) ? 1u : 0u;
+                c->n_new = 0;
+                c->prot = 0ull;
+                c->any_perfect = 0;
+                if (taken != need) c->error = 4u;
+                atomicAdd(&p_dbg_appends, static_cast<unsigned long long>(appended));
+            }
+        } else if (in) {
+            used = c->tail[b] - c->head[b];          // evict_tier wrote the counters (rare: a second round trip)
+        }
+        // per-batch scratch of the tier
+        const unsigned n_tk = min(ticket + nev, tier.lb_cap);
+        for (unsigned i = lane; i < n_tk; i += 32) tier.lookback[i] = 0ull;
+        c->kept[b] = ~0ull;
+        c->scan_end[b] = 0ull;
+        if (t == 0) {
+            p.tot[b] = 0u;
+        } else {
+            p.tot[kMaxBuckets + b] = 0u;
+            p.tot[2 * kMaxBuckets + b] = 0u;
+        }
+        if (lane == 0) {
+            c->ticket = 0;
+            c->done_ctas = 0;
+            c->stop = 0;
+            c->n_taken = 0;
+            if (t == 0) {
+                atomicAdd(&p.dbg[20], static_cast<unsigned long long>(ticket + nev));
+                atomicAdd(&p.dbg[21], total_v);
+            }
+        }
+#pragma unroll
+        for (int k = 16; k > 0; k >>= 1) {
+            const unsigned long long x = __shfl_xor_sync(kFull, used, k);
+            used = x > used ? x : used;
+        }
+    } else if (warp == kPhaseWarp) {
+        t5 = gtime();
+        d = __ldcg(&p.dbg[lane]);
+    }
+    // C3 reads both tiers' n_evicted_last
+    __syncthreads();
+    if (p.c3.active) c3_update(p);
+    if (warp == 0 && world > 1) {
+        // every row this rank owes its peers has been stored (k_serve's gather, the fetch role): tell them, then
+        // hold the stream until every peer has said the same to us
+        const ShardArgs *sh = &p.args->sh;
+        const unsigned epoch = sh->epoch;
+        __threadfence_system();
+        if (lane < world) *reinterpret_cast<volatile unsigned *>(sh->out_flag[lane]) = epoch;
+        const unsigned long long tw0 = gtime();
+        wait_flags(sh->my_out_flags, world, epoch, lane, p);
+        if (lane == 0) p.dbg[29] += gtime() - tw0;
+    }
+    // the host's view of the ring occupancy (maintain_rings): one 8-byte store into mapped pinned memory per tier, tagged
+    // with the batch number; nothing waits for it to land
+    if (warp < p.n_tiers && lane == 0)
+        *reinterpret_cast<volatile unsigned long long *>(p.ring_host + warp) =
+            (static_cast<unsigned long long>(seq) << 32) | (used & 0xFFFFFFFFull);
+    if (warp == kPhaseWarp) {
+        // phase accounting, one accumulator per lane, from the words loaded with the plans above:
+        // running sums over batches (ns): [8] serve, [9] gap, [10] update, [11] gap, [12] evict(+c3), [13] count;
+        // k_evict in detail: [22] plan, [23] chunk loops (slowest CTA), [24] wait for the last arrival, [25] close + C3
+        t5 = __shfl_sync(kFull, t5, 0);
+        unsigned long long t6 = (lane == 0) ? gtime() : 0ull;
+        t6 = __shfl_sync(kFull, t6, 0);
+        const unsigned long long v0 = __shfl_sync(kFull, d, 0), v1 = __shfl_sync(kFull, d, 1), v2 = __shfl_sync(kFull, d, 2),
+                                 v3 = __shfl_sync(kFull, d, 3), v4 = __shfl_sync(kFull, d, 4), v16 = __shfl_sync(kFull, d, 16),
+                                 v17 = __shfl_sync(kFull, d, 17);
+        const unsigned long long nv = lane == 5 ? t5 : lane == 6 ? t6 : lane == 7 ? v1 : lane == 8 ? d + (v1 - v0)
+                                    : lane == 9 ? d + (v2 - v1) : lane == 10 ? d + (v3 - v2) : lane == 11 ? d + (v4 - v3)
+                                    : lane == 12 ? d + (t6 - v4) : lane == 13 ? d + 1ull : lane == 18 ? t5
+                                    : lane == 22 ? d + (v16 - v4) : lane == 23 ? d + (v17 - v16) : lane == 24 ? d + (t5 - v17)
+                                    : d + (t6 - t5);
+        const bool wr = (lane >= 5 && lane <= 13) || lane == 18 || (lane >= 22 && lane <= 25);
+        if (wr) p.dbg[lane] = nv;
+        if (lane == 0) atomicAdd(&p.g->batches, 1ull);
+    }
+}
+
 // One launch, three kinds of CTA (blockIdx.y = role): roles 0 .. n_tiers-1 evict from that tier (p.evict_ctas CTAs each),
 // role n_tiers fetches the batch's missing rows (p.fetch_ctas CTAs: fetch_list_body, evs_kernels.cuh).  The two do not
 // depend on each other -- both follow k_update -- so they used to be two kernels on two streams joined by events;
 // as roles of one grid the batch is a linear chain of three launches (no fork / join inside the graph).
-// The last role to finish closes the batch: C3 insertions, and for a sharded handle the "my rows are delivered"
-// words to the peers and the wait for theirs.
+// The last CTA to arrive, of any role, closes the batch (close_batch): the tiers' counters, C3 insertions, and for a
+// sharded handle the "my rows are delivered" words to the peers and the wait for theirs.
 template <int P0, int P1>
 __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__ Params p) {
     extern __shared__ __align__(16) unsigned char s_stage[];    // fetch role: warps * max(row_stride); unaligned rows only
@@ -444,7 +570,7 @@ __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__
         if (p.dbg[0] > p.dbg[2]) p.dbg[14] += 1000ull;      // the next batch's k_serve already started (must not happen)
     }
 
-    // ---- plan: lane = bucket --------------------------------------------------------------
+    // ---- plan: lane = bucket; every input in one round of independent loads ----------------
     if (warp == 0) {
         const int b = lane;
         const bool in = b < tier.n_buckets;
@@ -455,13 +581,15 @@ __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__
         const unsigned cnt = in ? c->count[b] : 0u;
         const unsigned n_new = c->n_new;
         const unsigned long long prot = c->prot;
+        const unsigned n_perfect = c->n_perfect;
+        const unsigned any_perfect = c->any_perfect;
         unsigned size = cnt, appended = app;
 #pragma unroll
         for (int d = 16; d > 0; d >>= 1) {
             size += __shfl_xor_sync(kFull, size, d);
             appended += __shfl_xor_sync(kFull, appended, d);
         }
-        const int prot_b = n_new ? static_cast<int>(prot >> 32) - 1 : -1;
+        const int prot_b = n_new ? prot_bucket(prot) : -1;
         const unsigned need = size > tier.cap ? size - tier.cap : 0u;
         const unsigned avail = cnt - ((b == prot_b && cnt > 0) ? 1u : 0u);
         unsigned incl = avail;
@@ -490,24 +618,41 @@ __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__
             P.seg_off[si] = lincl - len;
         }
         const unsigned long long total_v = __shfl_sync(kFull, lincl, 31);
+        const unsigned top_left = __shfl_sync(kFull, cnt - take, top);
+        const bool overflow = total_v > static_cast<unsigned long long>(tier.lb_cap) * W;     // cannot happen unless a ring overflowed
+        const unsigned flush = (n_new > 0 && n_perfect >= tier.max_perfect) ? 1u : 0u;
         if (lane == 0) {
             const int n = __popc(has);
             P.n_seg = n;
             P.seg_off[n] = total_v;
             P.size = size;
-            P.need = need;
-            if (total_v > static_cast<unsigned long long>(tier.lb_cap) * W) {     // cannot happen unless a ring overflowed
-                c->error = 5u;
-                P.need = 0;
-            }
+            P.need = overflow ? 0u : need;
+            if (overflow) c->error = 5u;
             P.n_new = n_new;
-            P.n_perfect = c->n_perfect;
-            P.any_perfect = c->any_perfect;
-            P.flush = (n_new > 0 && c->n_perfect >= tier.max_perfect) ? 1u : 0u;
+            P.n_perfect = n_perfect;
+            P.any_perfect = any_perfect;
+            P.flush = flush;
             P.prot_b = prot_b;
-            P.prot_slot = n_new ? (__ldcg(p.pos_slot + static_cast<unsigned>(prot & 0xFFFFFFFFull)) & ~kClaimedBit) : kNoSlot;
+            P.prot_slot = n_new ? prot_slot(prot) : kNoSlot;
             P.appended = appended;
             s_taken = 0;
+        }
+        if (blockIdx.x == 0) {
+            // the plan, for whichever CTA closes the batch (close_batch)
+            EvictOut &o = ctl->out;
+            o.head[b] = head;
+            o.tail[b] = tail;
+            o.count[b] = cnt - take;
+            if (lane == 0) {
+                o.total_v = total_v;
+                o.take_mask = has;
+                o.size = size;
+                o.need = overflow ? 0u : need;
+                o.top_left = top_left;
+                o.any_perfect = any_perfect;
+                o.flush = flush;
+                o.appended = appended;
+            }
         }
     }
     __syncthreads();
@@ -524,6 +669,8 @@ __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__
             if (threadIdx.x < tier.n_buckets) c->tail[threadIdx.x] = P.tail[threadIdx.x];
             __syncthreads();
             evict_tier(tier, p);
+        } else if (threadIdx.x == 0) {
+            atomicAdd(&ctl->done_ctas, 1u);
         }
     } else if (P.need > 0) {
         const unsigned need = P.need;
@@ -601,7 +748,8 @@ __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__
                 evict_slot(tier, slot, key);
                 tier.evicted[before + idx] = key;
             }
-            // first live record left in place, per bucket: within a warp q grows with the lane
+            // first live record left in place, per bucket: within a warp q grows with the lane.  The plain pre-check keeps
+            // the same-address atomics few (a bare atomicMin from every warp measured no faster)
             const bool stays = live && !takeit;
             unsigned pending = __ballot_sync(kFull, stays);
             while (pending) {
@@ -623,131 +771,26 @@ __global__ void __launch_bounds__(kEvictThreads) k_evict(const __grid_constant__
         }
     }
 
-    // ---- the last CTA of the tier writes the tier's counters back ---------------------------
+    // ---- arrival ----------------------------------------------------------------------------
     __syncthreads();
     if (t == 0 && threadIdx.x == 0) atomicMax(&p.dbg[17], gtime());
-    if (threadIdx.x == 0) {
-        if (s_taken) atomicAdd(&ctl->n_taken, s_taken);
-        __threadfence();
-        s_last = (atomicAdd(&ctl->done_ctas, 1u) == nev - 1) ? 1u : 0u;
-    }
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    if (t == 0 && threadIdx.x == 0) {
-        p.dbg[18] = gtime();
-        p.dbg[20] += c->ticket + nev;
-        p.dbg[21] += P.seg_off[P.n_seg];
-    }
-    if (!P.flush) {
-        const unsigned taken = c->n_taken;
-        if (threadIdx.x < tier.n_buckets) {
-            const int b = threadIdx.x;
-            const unsigned cnt = P.count[b] - P.take[b];
-            unsigned long long head = P.head[b];
-            if (P.take[b] > 0) {
-                const unsigned long long kept = c->kept[b], se = c->scan_end[b];
-                head = (kept != ~0ull) ? kept : (se > head ? se : head);
-            }
-            if (cnt == 0) head = P.tail[b];
-            if (P.tail[b] - head > tier.ring_cap) c->error = 4u;
-            c->head[b] = head;
-            c->tail[b] = P.tail[b];
-            c->count[b] = cnt;
-        }
-        if (threadIdx.x == 0) {
-            const unsigned size = P.size - taken;
-            if (P.any_perfect) c->n_perfect = P.count[top] - P.take[top];       // EvLFU_C1.py:163-165
-            c->stat_evictions += taken;
-            c->n_evicted_last = taken;
-            c->n_flushed_last = 0;
-            c->full_at_start = (size >= tier.cap) ? 1u : 0u;
-            c->n_new = 0;
-            c->prot = 0ull;
-            c->any_perfect = 0;
-            if (taken != P.need) c->error = 4u;
-            atomicAdd(&p_dbg_appends, static_cast<unsigned long long>(P.appended));
-        }
-    }
-    // the host's view of the ring occupancy (maintain_rings): one 8-byte store into mapped pinned memory
-    __syncthreads();
-    if (warp == 0) {
-        unsigned long long used = 0ull;
-        if (lane < tier.n_buckets) used = c->tail[lane] - c->head[lane];
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            const unsigned long long o = __shfl_xor_sync(kFull, used, d);
-            used = o > used ? o : used;
-        }
-        if (lane == 0)
-            *reinterpret_cast<volatile unsigned long long *>(p.ring_host + t) =
-                (static_cast<unsigned long long>(p.args->seq) << 32) | (used & 0xFFFFFFFFull);
-    }
-    // per-batch scratch of the tier
-    const unsigned n_tk = min(c->ticket + nev, tier.lb_cap);
-    for (unsigned i = threadIdx.x; i < n_tk; i += blockDim.x) tier.lookback[i] = 0ull;
-    if (threadIdx.x < kMaxBuckets) {
-        c->kept[threadIdx.x] = ~0ull;
-        c->scan_end[threadIdx.x] = 0ull;
-        if (t == 0) {
-            p.tot[threadIdx.x] = 0u;
-        } else {
-            p.tot[kMaxBuckets + threadIdx.x] = 0u;
-            p.tot[2 * kMaxBuckets + threadIdx.x] = 0u;
-        }
-    }
-    if (threadIdx.x == 0) {
-        c->ticket = 0;
-        c->done_ctas = 0;
-        c->stop = 0;
-        c->n_taken = 0;
-    }
+    if (threadIdx.x == 0 && s_taken) atomicAdd(&ctl->n_taken, s_taken);
 
     }   // eviction role
 
-    // ---- the last role to finish feeds C3 and closes the batch ------------------------------------
+    // ---- one arrival level: every eviction CTA of every tier and the last fetch CTA; the last to arrive closes the batch
     __syncthreads();
     if (threadIdx.x == 0) {
         __threadfence();
+        const unsigned n_arrivals = static_cast<unsigned>(p.n_tiers * p.evict_ctas) + 1u;
         const unsigned prev = atomicAdd(p.done, 1u);
-        s_last = (prev == static_cast<unsigned>(p.n_tiers)) ? 1u : 0u;
+        s_last = (prev == n_arrivals - 1u) ? 1u : 0u;
         if (s_last) *p.done = 0u;
     }
     __syncthreads();
     if (!s_last) return;
     __threadfence();
-    if (threadIdx.x == 0) p.dbg[5] = gtime();
-    if (p.c3.active) c3_update(p);
-    if (warp == 0 && p.args->sh.world > 1) {
-        // every row this rank owes its peers has been stored (k_serve's gather, the fetch role): tell them, then
-        // hold the stream until every peer has said the same to us
-        const ShardArgs *sh = &p.args->sh;
-        const int world = sh->world;
-        const unsigned epoch = sh->epoch;
-        __threadfence_system();
-        if (lane < world) *reinterpret_cast<volatile unsigned *>(sh->out_flag[lane]) = epoch;
-        const unsigned long long tw0 = gtime();
-        wait_flags(sh->my_out_flags, world, epoch, lane, p);
-        if (lane == 0) p.dbg[29] += gtime() - tw0;
-    }
-    if (warp == 0) {
-        // phase accounting, one accumulator per lane (a single round trip at the very end of the batch):
-        // running sums over batches (ns): [8] serve, [9] gap, [10] update, [11] gap, [12] evict(+c3), [13] count;
-        // k_evict in detail: [22] plan, [23] chunk loops (slowest CTA), [24] wait for the last CTA, [25] write-back + C3
-        unsigned long long t6 = (lane == 0) ? gtime() : 0ull;
-        t6 = __shfl_sync(kFull, t6, 0);
-        const unsigned long long d = __ldcg(&p.dbg[lane]);
-        const unsigned long long v0 = __shfl_sync(kFull, d, 0), v1 = __shfl_sync(kFull, d, 1), v2 = __shfl_sync(kFull, d, 2),
-                                 v3 = __shfl_sync(kFull, d, 3), v4 = __shfl_sync(kFull, d, 4), v16 = __shfl_sync(kFull, d, 16),
-                                 v17 = __shfl_sync(kFull, d, 17), v18 = __shfl_sync(kFull, d, 18);
-        const unsigned long long nv = lane == 6 ? t6 : lane == 7 ? v1 : lane == 8 ? d + (v1 - v0) : lane == 9 ? d + (v2 - v1)
-                                    : lane == 10 ? d + (v3 - v2) : lane == 11 ? d + (v4 - v3) : lane == 12 ? d + (t6 - v4)
-                                    : lane == 13 ? d + 1ull : lane == 22 ? d + (v16 - v4) : lane == 23 ? d + (v17 - v16)
-                                    : lane == 24 ? d + (v18 - v17) : d + (t6 - v18);
-        const bool wr = (lane >= 6 && lane <= 13) || (lane >= 22 && lane <= 25);
-        if (wr) p.dbg[lane] = nv;
-        if (lane == 0) atomicAdd(&p.g->batches, 1ull);
-    }
+    close_batch(p);
 }
 
 }  // namespace evs
