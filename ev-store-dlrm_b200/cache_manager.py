@@ -330,15 +330,9 @@ class EvStore:
         _native.check(self.lib.evs_wait_host(self.handle, ticket), "evs_wait_host")
 
     def interact(self, x, ly, out=None, stream=None):
-        """dlrm interact_features (dot): x [B, d], ly [B, n_f, d] -> [B, d + (n_f+1) n_f / 2]."""
-        import torch
-        B, d = x.shape
-        n_f = ly.shape[1]
-        if out is None:
-            out = torch.empty((B, d + (n_f + 1) * n_f // 2), dtype=torch.float32, device=x.device)
-        st = _stream_handle(stream, x.device)
-        _native.check(self.lib.evs_interact(x.data_ptr(), ly.data_ptr(), out.data_ptr(), B, n_f, d, st), "evs_interact")
-        return out
+        """dlrm interact_features (dot): x [B, d], ly [B, n_f, d] -> [B, d + (n_f+1) n_f / 2] (dlrm_ops.interact_features)."""
+        from . import dlrm_ops
+        return dlrm_ops.interact_features(x, ly, out=out, stream=stream)
 
     def store_ptr(self, table: int, tier: int = 0):
         """(device-visible pointer, precision) of the backing rows of a table (evs_store_ptr)."""

@@ -9,9 +9,10 @@
 //     unchanged, as the "column-major" B operand (B[k][n] = T[n][k]), so a lane loads 8 values per k-step and uses
 //     them for both.  Only the 6 of 8 accumulator tiles that touch the strict lower triangle are computed;
 //   * fp32 accuracy from TF32 hardware: every operand is split hi + lo (hi = the value rounded to TF32's mantissa, lo = the
-//     rounded remainder) and a tile is the sum of hi*hi + hi*lo + lo*hi (the "3xTF32" scheme; the dropped lo*lo term is
-//     2^-22 relative).  The kernel is bound
-//     by HBM (7-11 FLOP/B), so the 3x tensor work is free;
+//     exact remainder, which the tensor core truncates to TF32) and a tile is the sum of hi*hi + hi*lo + lo*hi (the
+//     "3xTF32" scheme: the dropped lo*lo term and lo's truncation are 5 * 2^-22 relative together).  NaN and Inf inputs
+//     give NaN pairs (lo = v - hi is NaN for both); a finite value within 2^-11 of FLT_MAX rounds to hi = Inf and gives
+//     NaN as well.  The kernel is bound by issue slots (7-11 FLOP/B), so the 3x tensor work is free;
 //   * the accumulators go back through shared memory so that the 351 packed outputs are written as consecutive floats.
 // k_interact (fp32 FMA) remains for shapes outside those limits.
 #pragma once
@@ -19,17 +20,17 @@
 
 namespace evs {
 
-constexpr int kInteractWarps = 4;
+constexpr int kInteractWarps = 4;            // at most; fewer when (n_f + 1) (d + 1) floats per warp do not fit 4 times
 
 __global__ void __launch_bounds__(kInteractWarps * 32) k_interact(const float *__restrict__ x, const float *__restrict__ ly,
                                                                   float *__restrict__ r, int B, int n_f, int D) {
     extern __shared__ float s_t[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
     const int nt = n_f + 1, ld = D + 1;
     float *t = s_t + static_cast<size_t>(warp) * nt * ld;
     const int n_pairs = nt * (nt - 1) / 2;
     const int out_w = D + n_pairs;
-    for (int s = blockIdx.x * kInteractWarps + warp; s < B; s += gridDim.x * kInteractWarps) {
+    for (int s = blockIdx.x * wpc + warp; s < B; s += gridDim.x * wpc) {
         const float *xs = x + static_cast<size_t>(s) * D;
         const float *ls = ly + static_cast<size_t>(s) * n_f * D;
         float *rs = r + static_cast<size_t>(s) * out_w;
@@ -200,12 +201,14 @@ __global__ void __launch_bounds__(kMmaWarps * 32, 3) k_interact_mma(const float 
             for (int j = 0; j < 4; ++j) {
                 // hi = the value rounded to TF32's 10 mantissa bits with two integer instructions (add half an ulp, mask):
                 // cvt.rna.tf32 runs at a quarter of the ALU rate, and at d = 64 its 256 conversions per sample were the
-                // longest pipe.  lo = the exact remainder, rounded the same way: |v - hi - lo| <= 2^-22 |v|, as with cvt.rna
+                // longest pipe.  lo = v - hi is exact and goes in unrounded: the tensor core ignores its low 13 bits, so
+                // |v - hi - lo_tf32| < 2^-21 |v|.  Rounding lo as well would halve that, but the add can carry a NaN's
+                // mantissa into the sign bit (0x7FFFFFFF -> -0.0): hi of a NaN may be +-0 or Inf, and lo must stay NaN
                 const float2 v = *reinterpret_cast<const float2 *>(tl + 8 * j * ld + k0);
                 hi[j][0] = (__float_as_uint(v.x) + 0x1000u) & 0xFFFFE000u;
-                lo[j][0] = (__float_as_uint(v.x - __uint_as_float(hi[j][0])) + 0x1000u) & 0xFFFFE000u;
+                lo[j][0] = __float_as_uint(v.x - __uint_as_float(hi[j][0]));
                 hi[j][1] = (__float_as_uint(v.y) + 0x1000u) & 0xFFFFE000u;
-                lo[j][1] = (__float_as_uint(v.y - __uint_as_float(hi[j][1])) + 0x1000u) & 0xFFFFE000u;
+                lo[j][1] = __float_as_uint(v.y - __uint_as_float(hi[j][1]));
             }
             // tile (m, n): rows 16m .. 16m+15 (A from row groups 2m, 2m+1), cols 8n .. 8n+7 (B from row group n)
 #define EVS_TILE(ti, m, n)                                                                                           \
@@ -265,6 +268,7 @@ inline int launch_interact(const float *x, const float *ly, float *r, int B, int
         if (smem > 48 * 1024) {
             cudaError_t e = cudaFuncSetAttribute(k_interact_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
             if (e != cudaSuccess) {
+                cudaGetLastError();                         // not left behind for the caller's next launch check
                 set_error(std::string("k_interact_mma smem: ") + cudaGetErrorString(e));
                 return EVS_ERR_CUDA;
             }
@@ -276,16 +280,30 @@ inline int launch_interact(const float *x, const float *ly, float *r, int B, int
         EVS_CUDA(cudaGetLastError());
         return EVS_OK;
     }
-    const size_t smem = static_cast<size_t>(kInteractWarps) * (n_f + 1) * (D + 1) * sizeof(float);
+    // the fp32 FMA kernel: a warp stages its sample's T in (n_f + 1) (d + 1) floats; as many warps per CTA (4 down to 1)
+    // as the device's opt-in shared memory holds
+    int dev = 0, optin = 0;
+    EVS_CUDA(cudaGetDevice(&dev));
+    EVS_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    const size_t per_warp = static_cast<size_t>(n_f + 1) * (D + 1) * sizeof(float);
+    if (per_warp > static_cast<size_t>(optin)) {
+        set_error("evs_interact: n_f = " + std::to_string(n_f) + ", dim = " + std::to_string(D) + " stages " +
+                  std::to_string(per_warp) + " B of shared memory per sample, more than the device's limit of " +
+                  std::to_string(optin) + " B per block");
+        return EVS_ERR_INVALID;
+    }
+    const int warps = static_cast<int>(std::min<size_t>(kInteractWarps, optin / per_warp));
+    const size_t smem = warps * per_warp;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_interact, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) {
+            cudaGetLastError();
             set_error(std::string("k_interact smem: ") + cudaGetErrorString(e));
             return EVS_ERR_CUDA;
         }
     }
-    const int ctas = std::min((B + kInteractWarps - 1) / kInteractWarps, 148 * 8);
-    k_interact<<<ctas, kInteractWarps * 32, smem, st>>>(x, ly, r, B, n_f, D);
+    const int ctas = static_cast<int>(std::min<long long>((static_cast<long long>(B) + warps - 1) / warps, 148 * 8));
+    k_interact<<<ctas, warps * 32, smem, st>>>(x, ly, r, B, n_f, D);
     EVS_CUDA(cudaGetLastError());
     return EVS_OK;
 }

@@ -90,22 +90,54 @@ def apply_emb_ori_dlrm(lS_o, lS_i, emb_l, v_W_l=None):
     return ly
 
 
+def _check_fp32_cuda(name, t, dims, device=None):
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise ValueError(f"interact_features: {name} must be a tensor, not {type(t).__name__}")
+    if t.dtype != torch.float32:
+        raise ValueError(f"interact_features: {name} must be float32, not {t.dtype}")
+    if not t.is_cuda or (device is not None and t.device != device):
+        raise ValueError(f"interact_features: {name} is on {t.device}, the interaction runs on {device or 'a CUDA device'}")
+    if t.dim() != dims:
+        raise ValueError(f"interact_features: {name} must have {dims} dimensions, not shape {tuple(t.shape)}")
+
+
 def interact_features(x, ly, out=None, stream=None):
-    """x [B, d], ly: list of n_f tensors [B, d] (or one [B, n_f, d] tensor) -> [B, d + (n_f+1) n_f / 2]."""
+    """x [B, d], ly: list of n_f tensors [B, d] (or one [B, n_f, d] tensor) -> [B, d + (n_f+1) n_f / 2].
+    Everything is float32 on one CUDA device; `out`, when given, must be a contiguous [B, d + (n_f+1) n_f / 2] tensor.
+    A list of views ``buf[:, k, :]`` of one contiguous [B, n_f, d] buffer (what apply_emb_evstore returns) is read in
+    place; any other list is stacked into one first."""
     import torch
     lib = _native.load_library()
+    _check_fp32_cuda("x", x, 2)
+    B, d = x.shape
     if isinstance(ly, (list, tuple)):
-        base = ly[0]._base if ly[0]._base is not None else None
+        if not ly:
+            raise ValueError("interact_features: ly is an empty list")
+        for k, t in enumerate(ly):
+            _check_fp32_cuda(f"ly[{k}]", t, 2, x.device)
+            if tuple(t.shape) != (B, d):
+                raise ValueError(f"interact_features: ly[{k}] has shape {tuple(t.shape)}, x has {(B, d)}")
         n_f = len(ly)
-        same = base is not None and base.dim() == 3 and base.shape[1] == n_f and base.is_contiguous() and all(
-            t._base is base and t.data_ptr() == base.data_ptr() + k * base.shape[2] * 4 for k, t in enumerate(ly))
+        base = ly[0]._base
+        same = base is not None and tuple(base.shape) == (B, n_f, d) and base.is_contiguous() and all(
+            t._base is base and t.stride() == (n_f * d, 1) and t.data_ptr() == base.data_ptr() + k * d * 4
+            for k, t in enumerate(ly))
         lyt = base if same else torch.stack(list(ly), dim=1).contiguous()
     else:
+        _check_fp32_cuda("ly", ly, 3, x.device)
+        if ly.shape[0] != B or ly.shape[2] != d:
+            raise ValueError(f"interact_features: ly has shape {tuple(ly.shape)}, x has {(B, d)}: want [{B}, n_f, {d}]")
         lyt = ly.contiguous()
-    B, d = x.shape
     n_f = lyt.shape[1]
+    want = (B, d + (n_f + 1) * n_f // 2)
     if out is None:
-        out = torch.empty((B, d + (n_f + 1) * n_f // 2), dtype=torch.float32, device=x.device)
+        out = torch.empty(want, dtype=torch.float32, device=x.device)
+    else:
+        _check_fp32_cuda("out", out, 2, x.device)
+        if tuple(out.shape) != want or not out.is_contiguous():
+            raise ValueError(f"interact_features: out must be a contiguous {want} tensor, not shape {tuple(out.shape)} "
+                             f"with strides {out.stride()}")
     st = _stream_handle(stream, x.device)
     _native.check(lib.evs_interact(x.contiguous().data_ptr(), lyt.data_ptr(), out.data_ptr(), B, n_f, d, st), "evs_interact")
     return out

@@ -236,6 +236,9 @@ int evs_dump_c3(evs_handle h, int64_t *keys, uint32_t *alt, uint8_t *recency, in
  *   x_dev  fp32 [B][dim]        bottom-MLP output
  *   ly_dev fp32 [B][n_f][dim]   pooled embeddings (evs_lookup_batch output)
  *   r_dev  fp32 [B][dim + (n_f+1)*n_f/2]   (arch_interaction_itself = 0)
+ * Pairs are fp32-accurate (DESIGN.md section 4); a NaN or +-Inf input makes every pair of its row NaN or non-finite.
+ * EVS_ERR_INVALID when one sample's (n_f+1) x (dim+1) floats exceed the device's shared memory per block (only for
+ * n_f + 1 > 32 or dim > 128).
  */
 int evs_interact(const float *x_dev, const float *ly_dev, float *r_dev, int32_t B, int32_t n_f, int32_t dim,
                  void *stream);

@@ -77,52 +77,6 @@ def test_ring_compaction_keeps_order(monkeypatch):
     run_single_tier_parity(SMALL_ROWS, 16, 32, 400, [64], 60, check_state_every=10, policy="lru")
 
 
-def test_interaction_matches_torch_bmm():
-    import torch
-    p = pkg()
-    tables = p.workload.make_tables(SMALL_ROWS, 16)
-    store = p.EvStore(tables, p.CacheConfig(total_size=300, max_batch=32))
-    # tensor cores (mma.sync TF32, hi + lo split) for n_f + 1 <= 32 and d <= 128; the fp32 FMA kernel for the last two
-    for B, nf, d in [(1, 26, 16), (37, 26, 36), (256, 26, 64), (5, 3, 8), (300, 31, 20), (9, 1, 4), (16, 26, 18), (5, 26, 128),
-                     (4, 32, 16), (3, 26, 160)]:
-        g = torch.Generator(device="cuda").manual_seed(B)
-        x = torch.randn((B, d), device="cuda", generator=g)
-        ly = torch.randn((B, nf, d), device="cuda", generator=g)
-        r = store.interact(x, ly)
-        T = torch.cat([x.unsqueeze(1), ly], dim=1)
-        Z = torch.bmm(T, T.transpose(1, 2))
-        li = torch.tensor([i for i in range(nf + 1) for j in range(i)])
-        lj = torch.tensor([j for i in range(nf + 1) for j in range(i)])
-        want = torch.cat([x, Z[:, li, lj]], dim=1)
-        # fp32 dot products, different summation order than cuBLAS: tolerance 1e-4 abs on O(d) sums
-        assert torch.allclose(r, want, rtol=1e-5, atol=1e-4), (B, nf, d)
-    store.close()
-
-
-def test_interaction_tensor_core_path_has_fp32_accuracy():
-    """The 3xTF32 split must not cost accuracy: against a float64 reference the tensor-core kernel is as close as
-    an fp32 bmm (a plain TF32 product would be off by ~1e-3 relative)."""
-    import torch
-    p = pkg()
-    torch.manual_seed(3)
-    B, n_f, d = 2048, 26, 64
-    x = torch.randn(B, d, device="cuda")
-    ly = torch.randn(B, n_f, d, device="cuda")
-    got = torch.empty((B, d + (n_f + 1) * n_f // 2), device="cuda")
-    torch.cuda.synchronize()
-    assert p.load_library().evs_interact(x.data_ptr(), ly.data_ptr(), got.data_ptr(), B, n_f, d, None) == 0
-    torch.cuda.synchronize()
-    T = torch.cat([x.unsqueeze(1), ly], dim=1).double()
-    Z = torch.bmm(T, T.transpose(1, 2))
-    li = torch.tensor([i for i in range(n_f + 1) for j in range(i)])
-    lj = torch.tensor([j for i in range(n_f + 1) for j in range(i)])
-    want = torch.cat([x.double(), Z[:, li, lj]], dim=1)
-    err = float((got.double() - want).abs().max())
-    ref32 = torch.bmm(T.float(), T.float().transpose(1, 2))[:, li, lj]
-    err32 = float((ref32.double() - want[:, d:]).abs().max())
-    assert err <= max(4 * err32, 2e-5), (err, err32)
-
-
 def test_back_to_back_batches_without_host_sync():
     """Batches queued back to back (no host synchronisation in between, as bench.py does): every
     batch must still see the state its predecessor left (stream order of the whole kernel graph)."""
