@@ -195,6 +195,53 @@ class EvStore:
         ev = ready_event.cuda_event if ready_event is not None else None
         _native.check(self.lib.evs_prefetch(self.handle, lS_i_next.data_ptr(), B, ev), "evs_prefetch")
 
+    def update_rows(self, tables, rows, values, stream=None):
+        """Refresh a model in service (evs_update_rows): new fp32 values for rows of the tables this store serves.
+
+        tables: a global table id (int) or an integer CUDA tensor [n] of them; rows: integer CUDA tensor [n];
+        values: float32 CUDA tensor [n, dim] (rows may be strided, elements contiguous).  Returns ``where``, a uint8 CUDA
+        tensor [n]: bit 0 = the C1 copy was refreshed, bit 1 = the C2 copy, bit 2 = the backing store was written,
+        0x80 = rejected (row out of range or table not served here -- which also makes ``check`` raise -- or a value the
+        stored precision cannot hold).  A key given twice takes its last row; the earlier occurrences report 0.
+
+        The backing store is written IN PLACE: with host backing rows that is the caller's own arrays -- for a 32-bit
+        store the fp32 tables passed to the constructor -- and, with ``store_in_hbm``, the HBM copy only.  Ordered on
+        ``stream`` (default: torch's current stream): lookups enqueued before see the old rows, lookups after the new
+        ones; cache contents, eviction order and statistics do not change.  Raises ValueError before any launch on a bad
+        dtype, device or shape."""
+        import torch
+        dev = torch.device("cuda", self.cfg.device)
+
+        def on_dev(x):
+            return torch.is_tensor(x) and x.is_cuda and x.device == dev
+
+        int_types = (torch.int64, torch.int32)
+        if not on_dev(rows) or rows.dtype not in int_types or rows.dim() != 1:
+            raise ValueError(f"rows must be a 1-D int64 / int32 tensor on {dev}")
+        n = int(rows.shape[0])
+        if not on_dev(values) or values.dtype != torch.float32 or values.dim() != 2 or tuple(values.shape) != (n, self.dim) \
+                or (n > 0 and self.dim > 1 and values.stride(1) != 1) or (n > 1 and values.stride(0) < self.dim):
+            raise ValueError(f"values must be a float32 tensor [{n}, {self.dim}] on {dev} with contiguous rows")
+        if torch.is_tensor(tables):
+            if not on_dev(tables) or tables.dtype not in int_types or tuple(tables.shape) != (n,):
+                raise ValueError(f"tables must be an int or a 1-D int64 / int32 tensor [{n}] on {dev}")
+            tab = tables.to(torch.int64)
+        elif isinstance(tables, (int, np.integer)):
+            tab = torch.full((n,), int(tables), dtype=torch.int64, device=dev)
+        else:
+            raise ValueError("tables must be an int or an integer CUDA tensor")
+        where = torch.empty((n,), dtype=torch.uint8, device=dev)
+        if n == 0:
+            return where
+        r = rows.to(torch.int64)
+        # (table << 40) | row; a negative table or row gives a negative key, which the library rejects
+        keys = torch.where((tab < 0) | (r < 0), torch.full_like(r, -1), (tab << 40) | r)
+        st = _stream_handle(stream, dev)
+        vstride = values.stride(0) if n > 1 else self.dim
+        rc = self.lib.evs_update_rows(self.handle, keys.data_ptr(), n, values.data_ptr(), vstride, where.data_ptr(), st)
+        _native.check(rc, "evs_update_rows")
+        return where
+
     def check(self, clear: bool = False):
         """Raise if a batch that has already run saw an out-of-range index or a silent peer (no synchronisation)."""
         _native.check(self.lib.evs_check(self.handle, int(clear)), "evs_check")

@@ -18,6 +18,7 @@
 #include "evs_prefetch.cuh"
 #include "evs_bags.cuh"
 #include "evs_knn.cuh"
+#include "evs_refresh.cuh"
 
 namespace evs {
 
@@ -318,6 +319,9 @@ static void free_all(evs_handle h) {
         for (void *p : h->tier[i].allocs) cudaFree(p);
     for (void *p : h->c3_allocs) cudaFree(p);
     for (void *p : h->dev_allocs) cudaFree(p);
+    if (h->upd_key) cudaFree(h->upd_key);
+    if (h->upd_pos) cudaFree(h->upd_pos);
+    if (h->ev_upd) cudaEventDestroy(h->ev_upd);
     release_host_ranges(h);
     h->prof.destroy();
     if (h->pf_stream) cudaStreamDestroy(h->pf_stream);
@@ -604,6 +608,26 @@ static int check_device_errors(evs_handle h) {
         }
     }
     return EVS_OK;
+}
+
+// k_update_rows by (main precision, secondary precision): evs_update_rows, evs_refresh.cuh
+using RefreshFn = void (*)(const Params, const RefreshArgs);
+template <int P0, int P1>
+static RefreshFn refresh_of() { return k_update_rows<P0, P1>; }
+static RefreshFn pick_refresh(int p0, int p1) {
+    switch (p0 * 100 + p1) {
+        case 3200: return refresh_of<32, 0>();
+        case 1600: return refresh_of<16, 0>();
+        case 800: return refresh_of<8, 0>();
+        case 400: return refresh_of<4, 0>();
+        case 3216: return refresh_of<32, 16>();
+        case 3208: return refresh_of<32, 8>();
+        case 3204: return refresh_of<32, 4>();
+        case 1608: return refresh_of<16, 8>();
+        case 1604: return refresh_of<16, 4>();
+        case 804: return refresh_of<8, 4>();
+        default: return nullptr;
+    }
 }
 
 }  // namespace evs
@@ -1166,6 +1190,81 @@ int evs_lookup_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev
             k_bags_pool<false><<<grid, 256, 0, st>>>(h->bag_rows, h->bag_hit, reinterpret_cast<const long long *>(off_dev), B, P, T, D, out_dev, os, hit_dev);
         EVS_CUDA(cudaGetLastError());
     }
+    return EVS_OK;
+}
+
+// New values for the rows of n keys (evs_refresh.cuh), stream-ordered between batches.
+int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const float *values_dev, int64_t value_stride,
+                    uint8_t *where_dev, void *stream) {
+    if (h == nullptr || n < 0 || value_stride < 0 || (value_stride > 0 && value_stride < h->cfg.dim) ||
+        (n > 0 && (keys_dev == nullptr || values_dev == nullptr))) {
+        set_error("evs_update_rows: bad handle / n / value_stride (0 or >= dim) / pointers");
+        return EVS_ERR_INVALID;
+    }
+    if (n == 0) return EVS_OK;
+    DeviceGuard dg(h->cfg.device);
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
+    {
+        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone) {
+            set_error("evs_update_rows: the stream is being captured; call it outside a graph, between launches");
+            return EVS_ERR_INVALID;
+        }
+    }
+    const RefreshFn fn = pick_refresh(h->tier[0].prec, h->n_tiers == 2 ? h->tier[1].prec : 0);
+    if (fn == nullptr) return EVS_ERR_INVALID;
+    if (n > (1ll << 30)) {
+        set_error("evs_update_rows: at most 2^30 keys per call");
+        return EVS_ERR_INVALID;
+    }
+    // scratch hash at a load factor <= 1/2; a larger call grows it synchronously (the previous call may still read it)
+    const size_t cap = next_pow2(static_cast<unsigned long long>(std::max<int64_t>(2 * n, 1024)));
+    if (cap > h->upd_cap) {
+        EVS_CUDA(cudaDeviceSynchronize());
+        if (h->upd_key) cudaFree(h->upd_key);
+        if (h->upd_pos) cudaFree(h->upd_pos);
+        h->upd_key = nullptr;
+        h->upd_pos = nullptr;
+        h->hbm_bytes -= h->upd_cap * (sizeof(unsigned long long) + sizeof(long long));
+        h->upd_cap = 0;
+        EVS_CUDA(cudaMalloc(&h->upd_key, cap * sizeof(unsigned long long)));
+        EVS_CUDA(cudaMalloc(&h->upd_pos, cap * sizeof(long long)));
+        h->upd_cap = cap;
+        h->hbm_bytes += cap * (sizeof(unsigned long long) + sizeof(long long));
+    }
+    if (h->ev_upd == nullptr) EVS_CUDA(cudaEventCreateWithFlags(&h->ev_upd, cudaEventDisableTiming));
+    RefreshArgs ra{};
+    ra.keys = reinterpret_cast<const long long *>(keys_dev);
+    ra.n = n;
+    ra.values = values_dev;
+    ra.vstride = value_stride > 0 ? value_stride : h->cfg.dim;
+    ra.where = where_dev;
+    ra.hkey = h->upd_key;
+    ra.hpos = h->upd_pos;
+    ra.hmask = static_cast<unsigned>(cap - 1);
+    ra.gsize = 1;
+    while (ra.gsize < 32 && 8 * ra.gsize < h->cfg.dim) ra.gsize <<= 1;
+    EVS_CUDA(cudaMemsetAsync(h->upd_key, 0xFF, cap * sizeof(unsigned long long), st));
+    EVS_CUDA(cudaMemsetAsync(h->upd_pos, 0xFF, cap * sizeof(long long), st));
+    void *args[] = {&h->params, &ra};
+    const long long per_cta = static_cast<long long>(kRefreshThreads / 32) * (32 / ra.gsize);
+    {
+        LaunchScope ls(h->prof, K_UPDATE_ROWS, st);
+        const unsigned g1 = static_cast<unsigned>(std::min<long long>((n + kRefreshThreads - 1) / kRefreshThreads, 148 * 16));
+        EVS_CUDA(launch_ex(reinterpret_cast<const void *>(k_update_rows_claim), dim3(g1), kRefreshThreads, 0, st, args, false));
+        // no programmatic serialization, here or in the claim: the next batch's k_serve (a programmatic dependent of
+        // whatever precedes it) cannot start before every row is written
+        const unsigned g2 = static_cast<unsigned>(std::min<long long>((n + per_cta - 1) / per_cta, 148 * 16));
+        EVS_CUDA(launch_ex(reinterpret_cast<const void *>(fn), dim3(g2), kRefreshThreads, 0, st, args, false));
+    }
+    // The look-ahead: an announcement made before this call may have staged old bytes (or may still be staging them).
+    // Cancel it -- the next batch fetches its misses itself; a k_prefetch still running tags its rows with a generation
+    // no later batch asks for -- and order every later k_prefetch behind the new bytes.
+    h->pf_seq = 0;
+    h->pf_idx = nullptr;
+    h->pf_B = 0;
+    EVS_CUDA(cudaEventRecord(h->ev_upd, st));
+    EVS_CUDA(cudaStreamWaitEvent(h->pf_stream, h->ev_upd, 0));
     return EVS_OK;
 }
 

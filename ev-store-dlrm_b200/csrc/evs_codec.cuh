@@ -37,6 +37,54 @@ __device__ __forceinline__ float dec4(unsigned v) {
     }
 }
 
+// Quantisers (evs_update_rows): bit-exact with codecs.encode_table / oracle/codecs.quantize_table, which evaluate
+// reduce_precision.py's expressions in float64 on float32 inputs.  Explicit _rn intrinsics keep nvcc from contracting
+// them into FMAs.  Each returns false for a value the format cannot hold, where numpy's astype would wrap silently.
+//   16-bit: trunc((v+0.65)/1.3*65000) inside +-0.65; outside, 65000 + trunc(+-100*(..)) made odd (negative) or even
+//           (positive); the code must land in [0, 65535] (|v| up to about 6)
+//   8-bit : rint((v+1)/2*254), round half to even; v must lie in [-1, 1]
+//   4-bit : searchsorted(side="right") over the edges: v == 0 (either sign) -> 7, -0.00025 <= v < 0 -> 8
+__device__ __forceinline__ bool enc16(float x, unsigned &q) {
+    if (!isfinite(x)) return false;
+    const double v = static_cast<double>(x);
+    double c;
+    if (v < -0.65) {
+        double b = trunc(__dmul_rn(-100.0, __dadd_rn(0.65, v)));
+        if (fmod(b, 2.0) == 0.0) b = __dadd_rn(b, 1.0);
+        c = __dadd_rn(65000.0, b);
+    } else if (v > 0.65) {
+        double t = trunc(__dmul_rn(100.0, __dsub_rn(v, 0.65)));
+        if (fmod(t, 2.0) == 1.0) t = __dsub_rn(t, 1.0);
+        c = __dadd_rn(65000.0, t);
+    } else {
+        c = trunc(__dmul_rn(__ddiv_rn(__dadd_rn(v, 0.65), 1.3), 65000.0));
+    }
+    if (!(c >= 0.0 && c <= 65535.0)) return false;
+    q = static_cast<unsigned>(c);
+    return true;
+}
+
+__device__ __forceinline__ bool enc8(float x, unsigned &q) {
+    if (!(x >= -1.0f && x <= 1.0f)) return false;          // NaN fails too
+    q = static_cast<unsigned>(rint(__dmul_rn(__ddiv_rn(__dadd_rn(static_cast<double>(x), 1.0), 2.0), 254.0)));
+    return true;
+}
+
+__device__ __forceinline__ bool enc4(float x, unsigned &q) {
+    if (!isfinite(x)) return false;
+    const double v = static_cast<double>(x);
+    if (v == 0.0) {
+        q = 7u;
+    } else if (v > 0.0) {
+        q = 6u - (v >= 0.00025) - (v >= 0.015) - (v >= 0.25) - (v >= 0.4) - (v >= 0.6) - (v >= 0.8);
+    } else if (v >= -0.00025) {
+        q = 8u;
+    } else {
+        q = 15u - (v >= -1.0) - (v >= -0.8) - (v >= -0.6) - (v >= -0.4) - (v >= -0.25) - (v >= -0.015);
+    }
+    return true;
+}
+
 // Shared-memory lookup tables for the byte codecs (filled once per CTA).
 struct CodecLut {
     float lut8[256];

@@ -38,9 +38,9 @@ struct Tier {
 
 
 // Kernel ids for the launch counter / per-kernel CUDA-event timing (evs_set_profiling).
-enum KernelId { K_SERVE = 0, K_SCAN, K_UPDATE, K_EVICT, K_PREFETCH, K_COMPACT, K_PROBE, K_INTERACT, K_GATHER, K_BAGS, K_COUNT };
+enum KernelId { K_SERVE = 0, K_SCAN, K_UPDATE, K_EVICT, K_PREFETCH, K_COMPACT, K_PROBE, K_INTERACT, K_GATHER, K_BAGS, K_UPDATE_ROWS, K_COUNT };
 static const char *const kKernelNames[K_COUNT] = {"k_serve", "k_scan", "k_update", "k_evict", "k_prefetch", "k_compact", "k_probe", "k_interact",
-                                                  "k_gather", "k_bags"};
+                                                  "k_gather", "k_bags", "k_update_rows"};
 
 struct Profiler {
     bool on = false;
@@ -140,6 +140,11 @@ struct evs_handle_s {
     long long *bag_idx = nullptr;
     float *bag_rows = nullptr;
     uint8_t *bag_hit = nullptr;
+    // evs_update_rows: scratch hash of one call's keys (grown, synchronously, when a call brings more keys)
+    unsigned long long *upd_key = nullptr;
+    long long *upd_pos = nullptr;
+    size_t upd_cap = 0;                      // entries of each (a power of two, >= 2 n)
+    cudaEvent_t ev_upd = nullptr;            // after the last update: orders the look-ahead stream behind it
     // staging for the host-buffer paths: slot 0 serves the synchronous call, all kPipeSlots the
     // pipelined one (H2D of batch n+1 and D2H of batch n-1 overlap the kernels of batch n)
     static constexpr int kPipeSlots = 4;

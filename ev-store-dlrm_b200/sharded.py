@@ -175,6 +175,23 @@ class ShardedLookup:
             res.append((ly.clone(), hit.clone()))         # lookup() reuses its buffers from call to call
         return res
 
+    def update_rows(self, tables, rows, values, stream=None):
+        """New values for rows of the model (``EvStore.update_rows``), called with the same arguments on every rank.
+        Each rank applies the entries of the tables it owns; no collective is needed, because a rank serves rows of its
+        own tables only.  Returns this rank's ``where`` [n]: the entries of other ranks' tables read 0."""
+        import torch
+        n = int(rows.shape[0])
+        where = torch.zeros((n,), dtype=torch.uint8, device=rows.device)
+        if torch.is_tensor(tables):
+            mine = torch.isin(tables, torch.as_tensor(self.my, dtype=tables.dtype, device=tables.device))
+        else:
+            mine = torch.full((n,), int(tables) in self.my, dtype=torch.bool, device=rows.device)
+        sel = mine.nonzero().flatten()
+        if sel.numel():
+            t = tables[sel] if torch.is_tensor(tables) else int(tables)
+            where[sel] = self.store.update_rows(t, rows[sel], values[sel], stream=stream)
+        return where
+
     def alltoall_bytes(self, B: int) -> int:
         """Bytes this rank sends to its peers per batch (SURVEY.md section 8(d))."""
         return B * self.T_local * self.dim * 4 * (self.world - 1) // self.world

@@ -15,6 +15,7 @@
  *        evs_lookup_batch / _batches / _bags / _batch_host / evs_submit_host   the hot path (device or host buffers,
  *                                                                      one batch, a queue of batches, bags with pooling)
  *        evs_prefetch, evs_note_replays                                look-ahead; the lookup inside a caller's CUDA graph
+ *        evs_update_rows                                               new row values, ordered between batches
  *        evs_shard_*                                                   table-wise sharding over NVLink peer memory
  *        evs_embedding_bag, evs_interact, evs_knn                      the ops either side of the cache; alt-key generation
  *        evs_host_alloc / evs_host_free                                host memory for backing rows (large device pages)
@@ -179,6 +180,26 @@ int evs_note_replays(evs_handle h, int64_t n, void *stream);
  *   ready_event  cudaEvent_t recorded after idx_dev was written, or NULL if the indices are already complete
  * Optional; a call that was not announced (or whose announcement does not match) runs as before. */
 int evs_prefetch(evs_handle h, const int64_t *idx_dev, int32_t B, void *ready_event);
+
+/* Refreshing a model in service: new fp32 values for the rows of n keys, written into the backing store at every
+ * precision the handle has (store_main / store_secondary: the caller's host arrays through the device mapping, or the HBM
+ * copy with store_in_hbm) and into every cached copy (the C1 / C2 slab row of a resident key).
+ *   keys_dev    int64 [n] in the library's key format, (global table << 40) | row (as evs_dump_state returns them)
+ *   values_dev  fp32 rows of dim floats, value_stride floats apart (0 = dim)
+ *   where_dev   uint8 [n] or NULL: bit 0 = the C1 copy was refreshed, bit 1 = the C2 copy, bit 2 = the backing store was
+ *               written; 0x80 = rejected, nothing written.  A key is rejected when its row is outside [0, rows[table]) or
+ *               its table is not served by this handle (this also raises the sticky EVS_ERR_INDEX of evs_check), or when a
+ *               quantised precision of the handle cannot hold one of its values: non-finite at 16 / 8 / 4 bits, outside
+ *               [-1, 1] at 8 bits, a 16-bit code outside [0, 65535] (|v| above about 6).  At 32 bits every bit pattern is
+ *               stored as given.  A key given several times takes the row of its LAST occurrence, whole; the earlier
+ *               occurrences write nothing and report 0 (the last one is still rejected on its own values).
+ * Stream-ordered: lookups enqueued on `stream` before the call see the old rows, lookups after it the new ones, whichever
+ * way a row is served (C1 / C2 / C3 / approximate substitution / miss / look-ahead, bags, evs_store_ptr readers).  The
+ * call changes no policy state (hit codes, buckets, eviction order, C3, statistics are what they would be without it);
+ * it cancels a pending evs_prefetch announcement, so the next batch fetches its misses itself.  Asynchronous; not
+ * allowed while `stream` is being captured (EVS_ERR_INVALID).  n == 0 is a no-op. */
+int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const float *values_dev, int64_t value_stride,
+                    uint8_t *where_dev, void *stream);
 
 /* Probe only: per-sample local hit counts (for the sharded exact mode the ranks
  * all-reduce these and pass the sum back as agg_in).  Does not change state. */
