@@ -401,11 +401,13 @@ static int maintain_rings(evs_handle h, int ti, cudaStream_t st, int ahead = 2) 
 using KernelFn = void (*)(const Params);
 using ServeFn = void (*)(const Params, const BatchArgs);
 using PrefetchFn = void (*)(const Params, const PrefetchArgs);
+using RefreshFn = void (*)(const Params, const RefreshArgs);
 struct KernelSet {
     ServeFn serve = nullptr;        // one GPU
     ServeFn serve_sh = nullptr;     // one rank of a table-wise sharded cache
     KernelFn evict = nullptr;       // eviction + miss-fetch roles
     PrefetchFn prefetch = nullptr;
+    RefreshFn update_rows = nullptr;   // evs_update_rows (evs_refresh.cuh)
 };
 template <int P0, int P1>
 static KernelSet kernels_of() {
@@ -414,6 +416,7 @@ static KernelSet kernels_of() {
     k.serve_sh = k_serve<P0, P1, true>;
     k.evict = k_evict<P0, P1>;
     k.prefetch = k_prefetch<P0, P1>;
+    k.update_rows = k_update_rows<P0, P1>;
     return k;
 }
 static KernelSet pick_kernels(int p0, int p1) {
@@ -507,14 +510,12 @@ static int build_graph_n(evs_handle h, int nb, cudaGraph_t *src_out, cudaGraphEx
     unsigned long long saved[K_COUNT];
     memcpy(saved, h->prof.launches, sizeof(saved));
     EVS_CUDA(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-    h->capturing = true;
     int rc = EVS_OK;
     for (int i = 0; i < nb && rc == EVS_OK; ++i) {
         BatchArgs none{};
         none.seq = kSeqMarker + static_cast<unsigned>(i);
         rc = enqueue_batch(h, h->stream, h->params.n_chunks_max, none, i > 0);
     }
-    h->capturing = false;
     cudaError_t e = cudaStreamEndCapture(h->stream, &g);
     memcpy(h->prof.launches, saved, sizeof(saved));
     h->prof.on = was_on;
@@ -608,26 +609,6 @@ static int check_device_errors(evs_handle h) {
         }
     }
     return EVS_OK;
-}
-
-// k_update_rows by (main precision, secondary precision): evs_update_rows, evs_refresh.cuh
-using RefreshFn = void (*)(const Params, const RefreshArgs);
-template <int P0, int P1>
-static RefreshFn refresh_of() { return k_update_rows<P0, P1>; }
-static RefreshFn pick_refresh(int p0, int p1) {
-    switch (p0 * 100 + p1) {
-        case 3200: return refresh_of<32, 0>();
-        case 1600: return refresh_of<16, 0>();
-        case 800: return refresh_of<8, 0>();
-        case 400: return refresh_of<4, 0>();
-        case 3216: return refresh_of<32, 16>();
-        case 3208: return refresh_of<32, 8>();
-        case 3204: return refresh_of<32, 4>();
-        case 1608: return refresh_of<16, 8>();
-        case 1604: return refresh_of<16, 4>();
-        case 804: return refresh_of<8, 4>();
-        default: return nullptr;
-    }
 }
 
 }  // namespace evs
@@ -919,51 +900,22 @@ static void count_batch_launches(evs_handle h) {
     if (h->params.n_chunks_max > h->params.quad_max) h->prof.launches[K_SCAN]++;
 }
 
-static int run_batch(evs_handle h, const BatchArgs &a_in, cudaStream_t st) {
-    const KernelSet ks = kernels_of_handle(h);
-    if (a_in.probe_only) {
-        LaunchScope ls(h->prof, K_PROBE, st);
-        EVS_CUDA(launch_serve(serve_of(h, ks), (a_in.B + h->params.spc - 1) / h->params.spc, st, h->params, a_in));
-        return EVS_OK;
-    }
-    // The caller is capturing its own graph (e.g. a whole sequential_forward): the batch goes in as plain kernels with frozen
-    // arguments; the device numbers each replay itself (BatchArgs::seq == 0) and the host is told by evs_note_replays.
-    {
-        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-        if (!h->capturing && cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive) {
-            BatchArgs a = a_in;
-            a.seq = 0u;
-            a.pf_gen = 0u;
-            return enqueue_batch(h, st, (a.B + h->params.spc - 1) / h->params.spc, a, false);
-        }
-    }
-    BatchArgs a = a_in;
-    const uint64_t seq = ++h->seq;
-    a.seq = static_cast<unsigned>(seq);
-    // rows staged by evs_prefetch are used when the announcement matches this call
-    a.pf_gen = (h->pf_ok && h->pf_seq == seq && h->pf_idx == static_cast<const void *>(a.idx) && h->pf_B == a.B) ? h->pf_gen : 0u;
-    if (h->use_graph && !h->prof.on) {
-        int rc = set_serve_params(h, h->graph, h->serve_node, a);
-        if (rc) return rc;
-        EVS_CUDA(cudaGraphLaunch(h->graph, st));
-        count_batch_launches(h);
-    } else {
-        // outside a graph the chain continues across batches: k_serve is a programmatic dependent of whatever kernel
-        // precedes it on the stream (the previous batch's k_evict in a serving loop)
-        int rc = enqueue_batch(h, st, (a.B + h->params.spc - 1) / h->params.spc, a, true);
-        if (rc) return rc;
-    }
-    // the staging rows of this parity may be overwritten (by the look-ahead for batch seq + 2) once this batch is done
-    if (h->pf_wait_mode == 1) {
-        EVS_CUDA(cudaEventRecord(h->ev_done[seq & 1], st));
-        h->ev_done_valid[seq & 1] = true;
-    }
-    h->batches++;
-    for (int i = 0; i < h->n_tiers; ++i) {
-        int rc = maintain_rings(h, i, st);
-        if (rc) return rc;
-    }
-    return EVS_OK;
+// CTAs of k_serve / k_update for B samples.
+static int serve_ctas(evs_handle h, int32_t B) { return (B + h->params.spc - 1) / h->params.spc; }
+
+// The stream a call is ordered on: the caller's, else the handle's own.
+static cudaStream_t stream_of(evs_handle h, void *stream) { return stream ? static_cast<cudaStream_t>(stream) : h->stream; }
+
+// The arguments of a lookup of B samples; out_stride <= 0: rows packed as [B][n_tables][dim].
+static BatchArgs lookup_args(evs_handle h, const int64_t *idx, int32_t B, float *out, int64_t out_stride, uint8_t *hit) {
+    BatchArgs a{};
+    a.idx = reinterpret_cast<const long long *>(idx);
+    a.B = B;
+    a.out = out;
+    a.out_stride = out_stride > 0 ? out_stride : static_cast<long long>(h->cfg.n_tables) * h->cfg.dim;
+    a.hit = hit;
+    a.agg_out = h->d_agg;
+    return a;
 }
 
 // Launch k_prefetch for batch number `seq` with generation `gen` on the look-ahead stream.  The kernel itself waits (on the
@@ -987,12 +939,12 @@ static int launch_prefetch(evs_handle h, const int64_t *idx_dev, int32_t B, uint
 
 // The next announcement's generation (tags are generation << 1 | tier: start over with clean tags before they wrap).
 static int next_pf_gen(evs_handle h, uint32_t *gen) {
-    if (++h->pf_gen >= 0x7FFFFFFFu) {
+    if (++h->pf.gen >= 0x7FFFFFFFu) {
         EVS_CUDA(cudaStreamSynchronize(h->stream));
         EVS_CUDA(cudaMemsetAsync(h->params.pf_tag, 0, 2 * sizeof(unsigned) * static_cast<size_t>(h->params.n_max), h->pf_stream));
-        h->pf_gen = 1;
+        h->pf.gen = 1;
     }
-    *gen = h->pf_gen;
+    *gen = h->pf.gen;
     return EVS_OK;
 }
 
@@ -1000,52 +952,128 @@ static int next_pf_gen(evs_handle h, uint32_t *gen) {
 static int prefetch_next(evs_handle h, const int64_t *idx_dev, int32_t B, cudaEvent_t ready) {
     if (!h->pf_ok) return EVS_OK;
     const uint64_t seq = h->seq + 1;
-    if (h->pf_seq == seq && h->pf_idx == static_cast<const void *>(idx_dev) && h->pf_B == B) return EVS_OK;   // already announced
+    if (h->pf.matches(seq, idx_dev, B)) return EVS_OK;   // already announced
     if (ready) EVS_CUDA(cudaStreamWaitEvent(h->pf_stream, ready, 0));
     if (h->pf_wait_mode == 1 && h->ev_done_valid[seq & 1]) EVS_CUDA(cudaStreamWaitEvent(h->pf_stream, h->ev_done[seq & 1], 0));
     uint32_t gen = 0;
     int rc = next_pf_gen(h, &gen);
     if (rc) return rc;
     if ((rc = launch_prefetch(h, idx_dev, B, seq, gen))) return rc;
-    h->pf_seq = seq;
-    h->pf_idx = idx_dev;
-    h->pf_B = B;
+    h->pf.record(seq, idx_dev, B);
     return EVS_OK;
 }
 
-// kGroup batches in ONE graph launch (evs_lookup_batches).  The batches stay strictly ordered -- the graph is the same
-// linear chain of kernels -- but only the first k_serve pays a graph-to-graph boundary; the others follow their
-// predecessor's k_evict over a programmatic edge.  The look-ahead kernels of batches 1 .. kGroup-1 are enqueued on the
-// look-ahead stream AFTER the graph (each waits on the device for the batch two before it, which is then already queued).
-static int run_group(evs_handle h, BatchArgs *a, int n, cudaStream_t st) {
-    const uint64_t seq0 = h->seq + 1;
-    uint32_t gens[evs_handle_s::kGroup] = {};
-    for (int i = 0; i < n; ++i) {
-        a[i].seq = static_cast<unsigned>(seq0 + i);
-        if (i == 0) {
-            a[i].pf_gen = (h->pf_ok && h->pf_seq == seq0 && h->pf_idx == static_cast<const void *>(a[i].idx) && h->pf_B == a[i].B) ? h->pf_gen : 0u;
-        } else if (h->pf_ok) {
-            int rc = next_pf_gen(h, &gens[i]);
-            if (rc) return rc;
-            a[i].pf_gen = gens[i];
-        }
-        int rc = set_serve_params(h, h->ggraph, h->gserve[i], a[i]);
-        if (rc) return rc;
-    }
-    EVS_CUDA(cudaGraphLaunch(h->ggraph, st));
-    h->seq += n;
-    for (int i = 0; i < n; ++i) count_batch_launches(h);
-    if (h->pf_ok) {
-        for (int i = 1; i < n; ++i) {
-            int rc = launch_prefetch(h, reinterpret_cast<const int64_t *>(a[i].idx), a[i].B, seq0 + i, gens[i]);
-            if (rc) return rc;
-        }
-        h->pf_seq = seq0 + n - 1;
-        h->pf_idx = a[n - 1].idx;
-        h->pf_B = a[n - 1].B;
-    }
-    h->batches += n;
+// A probe pass (evs_probe_batch, and the first pass of a sharded batch without the one-pass exchange): k_serve counts
+// every sample's hits and returns.  It is not a batch: no batch number, no bookkeeping, no ring appends.
+static int launch_probe(evs_handle h, BatchArgs a, cudaStream_t st) {
+    a.probe_only = 1;
+    LaunchScope ls(h->prof, K_PROBE, st);
+    EVS_CUDA(launch_serve(serve_of(h, kernels_of_handle(h)), serve_ctas(h, a.B), st, h->params, a));
     return EVS_OK;
+}
+
+// Submit a call's n consecutive batches of B samples on st: the one place that numbers batches, matches them with the
+// look-ahead and keeps the books.  fill(i, a) sets the arguments of batch i (a.idx = idx[i]) just before the batch is
+// submitted, in order; it may enqueue work on st ahead of the batch, and returns an error code.  may_group: the caller
+// allows h->group batches in one graph launch.
+extern "C++" {                                           // a template cannot have C linkage
+template <class Fill>
+static int submit_batches(evs_handle h, cudaStream_t st, int n, const int64_t *const *idx, int32_t B, bool may_group, Fill &&fill) {
+    // The caller is capturing its own graph (e.g. a whole sequential_forward): the batches go in as plain kernels with
+    // frozen arguments; the device numbers each replay itself (BatchArgs::seq == 0, pf_gen == 0) and the host is told by
+    // evs_note_replays.
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive) {
+        for (int i = 0; i < n; ++i) {
+            BatchArgs a{};
+            int rc = fill(i, a);
+            if (rc || (rc = enqueue_batch(h, st, serve_ctas(h, a.B), a, false))) return rc;
+        }
+        return EVS_OK;
+    }
+    const int G = h->group;
+    for (int i = 0; i < n;) {
+        // A group is one graph launch: the batches stay strictly ordered -- the graph is the same linear chain of kernels --
+        // but only the first k_serve pays a graph-to-graph boundary; the others follow their predecessor's k_evict over a
+        // programmatic edge.  Every bucket ring must take the whole group's appends (the host tracks an upper bound of the
+        // occupancy).
+        bool grouped = may_group && h->use_graph && !h->prof.on && G > 1 && h->ggraph != nullptr && h->pf_wait_mode == 0 && n - i >= G;
+        for (int t = 0; t < h->n_tiers && grouped; ++t) {
+            int rc = maintain_rings(h, t, st, G + 1);
+            if (rc) return rc;
+            grouped = ring_fits(h, t, G + 1);
+        }
+        const int m = grouped ? G : 1;
+        const uint64_t seq0 = h->seq + 1;
+        BatchArgs a[evs_handle_s::kGroup];
+        uint32_t gens[evs_handle_s::kGroup] = {};
+        for (int k = 0; k < m; ++k) {
+            a[k] = BatchArgs{};
+            int rc = fill(i + k, a[k]);
+            if (rc) return rc;
+            a[k].seq = static_cast<unsigned>(seq0 + k);
+            // rows staged by evs_prefetch are used when the announcement matches the batch; the later batches of a group
+            // are announced here, and their k_prefetch follows the graph launch
+            if (k == 0) {
+                a[k].pf_gen = h->pf.matches(seq0, a[k].idx, a[k].B) ? h->pf.gen : 0u;
+            } else if (h->pf_ok) {
+                if ((rc = next_pf_gen(h, &gens[k]))) return rc;
+                a[k].pf_gen = gens[k];
+            }
+        }
+        if (h->use_graph && !h->prof.on) {
+            const cudaGraphExec_t exec = grouped ? h->ggraph : h->graph;
+            for (int k = 0; k < m; ++k) {
+                int rc = set_serve_params(h, exec, grouped ? h->gserve[k] : h->serve_node, a[k]);
+                if (rc) return rc;
+            }
+            EVS_CUDA(cudaGraphLaunch(exec, st));
+            for (int k = 0; k < m; ++k) count_batch_launches(h);
+        } else {
+            // outside a graph the chain continues across batches: k_serve is a programmatic dependent of whatever kernel
+            // precedes it on the stream (the previous batch's k_evict in a serving loop)
+            int rc = enqueue_batch(h, st, serve_ctas(h, a[0].B), a[0], true);
+            if (rc) return rc;
+        }
+        h->seq += m;
+        h->batches += m;
+        if (grouped) {
+            if (h->pf_ok) {
+                for (int k = 1; k < m; ++k) {
+                    int rc = launch_prefetch(h, reinterpret_cast<const int64_t *>(a[k].idx), a[k].B, seq0 + k, gens[k]);
+                    if (rc) return rc;
+                }
+                h->pf.record(seq0 + m - 1, a[m - 1].idx, a[m - 1].B);
+            }
+        } else {
+            // the staging rows of this parity may be overwritten (by the look-ahead for batch seq + 2) once this batch is done
+            if (h->pf_wait_mode == 1) {
+                EVS_CUDA(cudaEventRecord(h->ev_done[seq0 & 1], st));
+                h->ev_done_valid[seq0 & 1] = true;
+            }
+            for (int t = 0; t < h->n_tiers; ++t) {
+                int rc = maintain_rings(h, t, st);
+                if (rc) return rc;
+            }
+            // the batch after it is announced so that its misses are staged as inside a group
+            if (i + 1 < n) {
+                int rc = prefetch_next(h, idx[i + 1], B, nullptr);
+                if (rc) return rc;
+            }
+        }
+        i += m;
+    }
+    return EVS_OK;
+}
+}  // extern "C++"
+
+// One batch whose arguments the caller built.
+static int submit_batch(evs_handle h, cudaStream_t st, const BatchArgs &a) {
+    const int64_t *idx = reinterpret_cast<const int64_t *>(a.idx);
+    return submit_batches(h, st, 1, &idx, a.B, false, [&](int, BatchArgs &b) {
+        b = a;
+        return EVS_OK;
+    });
 }
 
 int evs_prefetch(evs_handle h, const int64_t *idx_dev, int32_t B, void *ready_event) {
@@ -1065,17 +1093,9 @@ int evs_lookup_batch(evs_handle h, const int64_t *idx_dev, int32_t B, float *out
     }
     if (B == 0) return EVS_OK;
     DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
-    BatchArgs a{};
-    a.idx = reinterpret_cast<const long long *>(idx_dev);
-    a.out = out_dev;
-    a.out_stride = out_stride > 0 ? out_stride : static_cast<long long>(h->cfg.n_tables) * h->cfg.dim;
-    a.hit = hit_dev;
+    BatchArgs a = lookup_args(h, idx_dev, B, out_dev, out_stride, hit_dev);
     a.agg_in = agg_in;
-    a.agg_out = h->d_agg;
-    a.B = B;
-    a.probe_only = 0;
-    return run_batch(h, a, st);
+    return submit_batch(h, stream_of(h, stream), a);
 }
 
 int evs_lookup_batches(evs_handle h, int32_t n, const int64_t *const *idx_dev, int32_t B, float *const *out_dev, int64_t out_stride,
@@ -1090,43 +1110,10 @@ int evs_lookup_batches(evs_handle h, int32_t n, const int64_t *const *idx_dev, i
             return EVS_ERR_INVALID;
         }
     DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
-    const int G = h->group;
-    const unsigned long long n_max = static_cast<unsigned long long>(h->cfg.max_batch) * h->cfg.n_tables;
-    int i = 0;
-    while (i < n) {
-        bool grouped = h->use_graph && !h->prof.on && !h->sharded && G > 1 && h->ggraph != nullptr && n - i >= G && h->pf_wait_mode == 0;
-        if (grouped) {
-            // every bucket ring must take the whole group's appends (the host tracks an upper bound of the occupancy)
-            for (int t = 0; t < h->n_tiers && grouped; ++t) {
-                int rc = maintain_rings(h, t, st, G + 1);
-                if (rc) return rc;
-                grouped = ring_fits(h, t, G + 1);
-            }
-        }
-        if (grouped) {
-            BatchArgs a[evs_handle_s::kGroup];
-            for (int k = 0; k < G; ++k) {
-                a[k] = BatchArgs{};
-                a[k].idx = reinterpret_cast<const long long *>(idx_dev[i + k]);
-                a[k].out = out_dev[i + k];
-                a[k].out_stride = out_stride > 0 ? out_stride : static_cast<long long>(h->cfg.n_tables) * h->cfg.dim;
-                a[k].hit = hit_dev ? hit_dev[i + k] : nullptr;
-                a[k].agg_out = h->d_agg;
-                a[k].B = B;
-            }
-            int rc = run_group(h, a, G, st);
-            if (rc) return rc;
-            i += G;
-        } else {
-            // one graph per batch; the batch after it is announced so that its misses are staged as inside a group
-            int rc = evs_lookup_batch(h, idx_dev[i], B, out_dev[i], out_stride, hit_dev ? hit_dev[i] : nullptr, nullptr, st);
-            if (rc) return rc;
-            if (i + 1 < n && (rc = prefetch_next(h, idx_dev[i + 1], B, nullptr))) return rc;
-            i += 1;
-        }
-    }
-    return EVS_OK;
+    return submit_batches(h, stream_of(h, stream), n, idx_dev, B, !h->sharded, [&](int i, BatchArgs &a) {
+        a = lookup_args(h, idx_dev[i], B, out_dev[i], out_stride, hit_dev ? hit_dev[i] : nullptr);
+        return EVS_OK;
+    });
 }
 
 // Bags (pooling factor > 1) on the cached path: see evs_bags.cuh.
@@ -1147,7 +1134,7 @@ int evs_lookup_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev
     }
     if (B == 0) return EVS_OK;
     DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
+    cudaStream_t st = stream_of(h, stream);
     const int T = h->cfg.n_tables, D = h->cfg.dim, P = max_per_bag;
     if (h->bag_idx == nullptr) {                              // slice scratch, on first use
         t_alloc_bytes = &h->hbm_bytes;
@@ -1168,15 +1155,9 @@ int evs_lookup_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev
             h->params, reinterpret_cast<const long long *>(idx_dev), reinterpret_cast<const long long *>(off_dev), B, P, nnz, h->bag_idx);
         EVS_CUDA(cudaGetLastError());
     }
-    BatchArgs a{};
-    a.idx = h->bag_idx;
-    a.out = h->bag_rows;
-    a.out_stride = static_cast<long long>(T) * D;
-    a.hit = h->bag_hit;
-    a.agg_out = h->d_agg;
-    a.B = Bv;
+    BatchArgs a = lookup_args(h, reinterpret_cast<const int64_t *>(h->bag_idx), Bv, h->bag_rows, 0, h->bag_hit);
     a.bags = 1;
-    int rc = run_batch(h, a, st);
+    int rc = submit_batch(h, st, a);
     if (rc) return rc;
     {
         LaunchScope ls(h->prof, K_BAGS, st);
@@ -1203,7 +1184,7 @@ int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const floa
     }
     if (n == 0) return EVS_OK;
     DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
+    cudaStream_t st = stream_of(h, stream);
     {
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
         if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone) {
@@ -1211,7 +1192,7 @@ int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const floa
             return EVS_ERR_INVALID;
         }
     }
-    const RefreshFn fn = pick_refresh(h->tier[0].prec, h->n_tiers == 2 ? h->tier[1].prec : 0);
+    const RefreshFn fn = kernels_of_handle(h).update_rows;
     if (fn == nullptr) return EVS_ERR_INVALID;
     if (n > (1ll << 30)) {
         set_error("evs_update_rows: at most 2^30 keys per call");
@@ -1260,9 +1241,7 @@ int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const floa
     // The look-ahead: an announcement made before this call may have staged old bytes (or may still be staging them).
     // Cancel it -- the next batch fetches its misses itself; a k_prefetch still running tags its rows with a generation
     // no later batch asks for -- and order every later k_prefetch behind the new bytes.
-    h->pf_seq = 0;
-    h->pf_idx = nullptr;
-    h->pf_B = 0;
+    h->pf.cancel();
     EVS_CUDA(cudaEventRecord(h->ev_upd, st));
     EVS_CUDA(cudaStreamWaitEvent(h->pf_stream, h->ev_upd, 0));
     return EVS_OK;
@@ -1271,7 +1250,7 @@ int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const floa
 int evs_note_replays(evs_handle h, int64_t n, void *stream) {
     if (h == nullptr || n < 0) return EVS_ERR_INVALID;
     DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
+    cudaStream_t st = stream_of(h, stream);
     h->seq += static_cast<uint64_t>(n);
     h->batches += static_cast<uint64_t>(n);
     for (int i = 0; i < h->n_tiers; ++i) {
@@ -1285,13 +1264,11 @@ int evs_probe_batch(evs_handle h, const int64_t *idx_dev, int32_t B, uint8_t *ag
     if (h == nullptr || B < 0 || B > h->cfg.max_batch || idx_dev == nullptr || agg_out_dev == nullptr) return EVS_ERR_INVALID;
     if (B == 0) return EVS_OK;
     DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
     BatchArgs a{};
     a.idx = reinterpret_cast<const long long *>(idx_dev);
     a.agg_out = agg_out_dev;
     a.B = B;
-    a.probe_only = 1;
-    return run_batch(h, a, st);
+    return launch_probe(h, a, stream_of(h, stream));
 }
 
 // The device error word as the host sees it (the kernels mirror it into pinned memory): sticky until cleared.
@@ -1774,6 +1751,21 @@ static int shard_check(evs_shard s, const char *what, int32_t B) {
     return EVS_OK;
 }
 
+// n consecutive global batches on this rank: batch i takes the next exchange epoch and gets that epoch's receive buffer,
+// which out_dev[i] reports; without the one-pass exchange a probe pass goes ahead of each batch.  The receive buffers
+// rotate through kRecvBufs = 4, so a buffer is valid until four batches later.
+static int shard_submit(evs_shard s, cudaStream_t st, int32_t n, const int64_t *const *idx_dev, int32_t B, uint8_t *const *hit_dev,
+                        float **out_dev) {
+    evs_handle h = s->h;
+    return submit_batches(h, st, n, idx_dev, B, s->fused, [&](int i, BatchArgs &a) {
+        const unsigned epoch = ++s->epoch;
+        a = lookup_args(h, idx_dev[i], B, nullptr, 0, hit_dev ? hit_dev[i] : nullptr);
+        a.sh = shard_args(s, B, epoch);
+        out_dev[i] = reinterpret_cast<float *>(s->block + s->off_recv + (epoch % evs_shard_s::kRecvBufs) * s->recv_bytes);
+        return s->fused ? EVS_OK : launch_probe(h, a, st);
+    });
+}
+
 int evs_shard_lookup(evs_shard s, const int64_t *idx_dev, int32_t B, uint8_t *hit_dev, float **out_dev, void *stream) {
     if (idx_dev == nullptr || out_dev == nullptr) {
         set_error("evs_shard_lookup: null pointer");
@@ -1781,32 +1773,12 @@ int evs_shard_lookup(evs_shard s, const int64_t *idx_dev, int32_t B, uint8_t *hi
     }
     int rc = shard_check(s, "evs_shard_lookup", B);
     if (rc) return rc;
-    evs_handle h = s->h;
-    DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
-    const unsigned epoch = ++s->epoch;
-    BatchArgs a{};
-    a.idx = reinterpret_cast<const long long *>(idx_dev);
-    a.B = B;
-    a.agg_out = h->d_agg;
-    a.sh = shard_args(s, B, epoch);
-    if (!s->fused) {
-        a.probe_only = 1;
-        if ((rc = run_batch(h, a, st))) return rc;
-    }
-    a.probe_only = 0;
-    a.hit = hit_dev;
-    a.out = nullptr;
-    a.out_stride = static_cast<long long>(h->cfg.n_tables) * h->cfg.dim;
-    rc = run_batch(h, a, st);
-    if (rc) return rc;
-    *out_dev = reinterpret_cast<float *>(s->block + s->off_recv + (epoch % evs_shard_s::kRecvBufs) * s->recv_bytes);
-    return EVS_OK;
+    DeviceGuard dg(s->h->cfg.device);
+    return shard_submit(s, stream_of(s->h, stream), 1, &idx_dev, B, &hit_dev, out_dev);
 }
 
-// n consecutive global batches in one call (evs_lookup_batches for a rank of a sharded cache): groups of 4 batches go to
-// the device as one captured graph on every rank.  out_dev[i] receives this rank's buffer of batch i; the receive buffers
-// rotate through kRecvBufs = 4, so a buffer is valid until four batches later.
+// n consecutive global batches in one call (evs_lookup_batches for a rank of a sharded cache): with the one-pass exchange,
+// groups of 4 batches go to the device as one captured graph on every rank.
 int evs_shard_lookup_many(evs_shard s, int32_t n, const int64_t *const *idx_dev, int32_t B, uint8_t *const *hit_dev, float **out_dev,
                           void *stream) {
     if (n < 0 || (n > 0 && (idx_dev == nullptr || out_dev == nullptr))) {
@@ -1815,40 +1787,8 @@ int evs_shard_lookup_many(evs_shard s, int32_t n, const int64_t *const *idx_dev,
     }
     int rc = shard_check(s, "evs_shard_lookup_many", B);
     if (rc) return rc;
-    evs_handle h = s->h;
-    DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : h->stream;
-    const int G = h->group;
-    const unsigned long long n_max = static_cast<unsigned long long>(h->cfg.max_batch) * h->cfg.n_tables;
-    int i = 0;
-    while (i < n) {
-        bool grouped = s->fused && h->use_graph && !h->prof.on && G > 1 && h->ggraph != nullptr && n - i >= G && h->pf_wait_mode == 0;
-        for (int t = 0; t < h->n_tiers && grouped; ++t) {
-            if ((rc = maintain_rings(h, t, st, G + 1))) return rc;
-            grouped = ring_fits(h, t, G + 1);
-        }
-        if (grouped) {
-            BatchArgs a[evs_handle_s::kGroup];
-            for (int k = 0; k < G; ++k) {
-                const unsigned epoch = ++s->epoch;
-                a[k] = BatchArgs{};
-                a[k].idx = reinterpret_cast<const long long *>(idx_dev[i + k]);
-                a[k].B = B;
-                a[k].agg_out = h->d_agg;
-                a[k].sh = shard_args(s, B, epoch);
-                a[k].hit = hit_dev ? hit_dev[i + k] : nullptr;
-                a[k].out_stride = static_cast<long long>(h->cfg.n_tables) * h->cfg.dim;
-                out_dev[i + k] = reinterpret_cast<float *>(s->block + s->off_recv + (epoch % evs_shard_s::kRecvBufs) * s->recv_bytes);
-            }
-            if ((rc = run_group(h, a, G, st))) return rc;
-            i += G;
-        } else {
-            if ((rc = evs_shard_lookup(s, idx_dev[i], B, hit_dev ? hit_dev[i] : nullptr, &out_dev[i], st))) return rc;
-            if (i + 1 < n && (rc = prefetch_next(h, idx_dev[i + 1], B, nullptr))) return rc;
-            i += 1;
-        }
-    }
-    return EVS_OK;
+    DeviceGuard dg(s->h->cfg.device);
+    return shard_submit(s, stream_of(s->h, stream), n, idx_dev, B, hit_dev, out_dev);
 }
 
 int evs_shard_destroy(evs_shard s) {

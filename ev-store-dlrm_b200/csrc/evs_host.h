@@ -88,6 +88,19 @@ struct LaunchScope {
     }
 };
 
+// The look-ahead announcement (evs_prefetch): k_prefetch staged, or is staging, the misses of batch number `seq` on the
+// indices `idx` of B samples and tags their rows with generation `gen`.  Every announcement draws a new generation
+// (next_pf_gen), so the rows of a cancelled or superseded one never match a later batch.
+struct Announcement {
+    uint64_t seq = 0;                        // 0: none (batch numbers start at 1)
+    const void *idx = nullptr;
+    int B = 0;
+    uint32_t gen = 0;
+    bool matches(uint64_t s, const void *i, int b) const { return seq == s && idx == i && B == b; }
+    void record(uint64_t s, const void *i, int b) { seq = s, idx = i, B = b; }
+    void cancel() { record(0, nullptr, 0); }
+};
+
 }  // namespace evs
 
 struct evs_handle_s {
@@ -111,7 +124,6 @@ struct evs_handle_s {
     cudaGraphExec_t ggraph = nullptr;
     cudaGraphNode_t gserve[kGroup] = {};
     bool use_graph = true;
-    bool capturing = false;                  // enqueue_batch is being captured into the graph
     bool use_pdl = true;                     // the batch's kernels are chained by programmatic dependent launch
     int fetch_list_ctas = 8;                 // CTAs of the miss-fetch role (EVSTORE_B200_FETCH_LIST_CTAS overrides)
     int evict_ctas = evs::kTierCtas;         // CTAs of k_evict per tier (EVSTORE_B200_EVICT_CTAS overrides)
@@ -124,10 +136,7 @@ struct evs_handle_s {
     int pf_ctas = 16;
     int pf_mode = 0, pf_wait_mode = 0;       // experiment switches (EVSTORE_B200_PF_MODE / _PF_WAIT)
     uint64_t seq = 0;                        // batches started on this handle
-    uint64_t pf_seq = 0;                     // batch number the last evs_prefetch staged for
-    uint32_t pf_gen = 0;                     // generation of that announcement (tags of its staged rows)
-    const void *pf_idx = nullptr;
-    int pf_B = 0;
+    evs::Announcement pf;                    // the batch the last look-ahead staged for
     unsigned *err_host = nullptr;            // pinned, device-mapped: last device-side error code (0 = none)
     unsigned long long *ring_host = nullptr; // same block: per tier, batch number << 32 | longest ring window after that batch
     int sticky_error = 0;                    // first error evs_check saw

@@ -106,10 +106,48 @@ def test_replays_of_a_caller_captured_graph():
                 out, hit = store.lookup(torch.from_numpy(idx).cuda())
                 _agree(store, oracle, tables, idx, out, hit, f"single call after replay {it}")
             if it == 4:
-                idx = [trace.batch(B) for _ in range(3)]
+                idx = [trace.batch(B) for _ in range(5)]                 # one group of 4 and one single batch
                 outs, hits = store.lookup_many([torch.from_numpy(i).cuda() for i in idx])
-                for k in range(3):
+                for k in range(5):
                     _agree(store, oracle, tables, idx[k], outs[k], hits[k], f"grouped call after replay {it}, batch {k}")
+            _state(store, oracle, f"after replay {it}")
+    finally:
+        store.close()
+
+
+def test_replays_of_a_caller_captured_grouped_call():
+    """A graph the caller captured around lookup_many of 5 batches (outside a capture: one group and one single): every
+    batch goes in as plain kernels the device numbers itself, replay after replay; single and grouped calls follow."""
+    import torch
+    p, tables, store, oracle, trace = _open(SMALL_ROWS, 600, 64, seed=13)
+    B, n, T = 64, 5, len(SMALL_ROWS)
+    try:
+        first = trace.batch(B)                                     # warm-up outside the graph (also a batch)
+        out, hit = store.lookup(torch.from_numpy(first).cuda())
+        _agree(store, oracle, tables, first, out, hit, "warm-up")
+        s_idx = [torch.from_numpy(trace.batch(B)).cuda() for _ in range(n)]
+        s_out = [torch.empty((B, T, 16), dtype=torch.float32, device="cuda") for _ in range(n)]
+        s_hit = [torch.empty((B, T), dtype=torch.uint8, device="cuda") for _ in range(n)]
+        torch.cuda.synchronize()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            store.lookup_many(s_idx, outs=s_out, hits=s_hit)
+        for it in range(3):
+            idx = [trace.batch(B) for _ in range(n)]
+            for d, i in zip(s_idx, idx):
+                d.copy_(torch.from_numpy(i))
+            g.replay()
+            store.note_replays(n)
+            for k in range(n):
+                _agree(store, oracle, tables, idx[k], s_out[k], s_hit[k], f"replay {it}, batch {k}")
+            _state(store, oracle, f"replay {it}")
+            idx = trace.batch(B)
+            out, hit = store.lookup(torch.from_numpy(idx).cuda())
+            _agree(store, oracle, tables, idx, out, hit, f"single call after replay {it}")
+            idx = [trace.batch(B) for _ in range(n)]
+            outs, hits = store.lookup_many([torch.from_numpy(i).cuda() for i in idx])
+            for k in range(n):
+                _agree(store, oracle, tables, idx[k], outs[k], hits[k], f"grouped call after replay {it}, batch {k}")
             _state(store, oracle, f"after replay {it}")
     finally:
         store.close()

@@ -3,8 +3,8 @@
 trace are built once, then for every variant (a set of EVSTORE_B200_* environment variables, read by
 evs_create) a fresh EvStore is created, warmed with the same batches and timed over the same batches.
 
-    python tools/ab_bench.py "EVSTORE_B200_EVICT_MODE=0" "EVSTORE_B200_EVICT_MODE=1" \
-                             "EVSTORE_B200_EVICT_MODE=1,EVSTORE_B200_EVICT_CTAS=96"
+    python tools/ab_bench.py default "EVSTORE_B200_PDL=0" \
+                             "EVSTORE_B200_PDL=0,EVSTORE_B200_EVICT_CTAS=96"
 
 One JSON line per variant on stdout (value = lookups/s, device-resident indices, CUDA events).
 """
