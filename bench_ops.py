@@ -101,7 +101,8 @@ def bench_embedding_bag(pkg, dev, B=16384, P=10, d=64, rows=4_000_000, prec=32, 
 
 def bench_knn(pkg, dev, n=262144, d=16, K=3):
     """evs_knn, every row of an [n, d] matrix against all rows (the alt-key generator's inner loop).  FLOP = 2 d per pair (the
-    tensor cores execute 3x that for the hi / lo split); the kernel is bound by the selection's ALU work, not by the tensor pipe."""
+    tensor cores execute 3x that for the hi / lo split: hi rounded to TF32, lo the exact remainder, truncated by the tensor
+    core); the kernel is bound by the selection's ALU work, not by the tensor pipe."""
     import torch
     x = torch.randn((n, d), device=dev)
     nbr = pkg.altkeys.knn(x)                              # warm-up (and the result for the spot check)

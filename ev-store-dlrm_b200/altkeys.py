@@ -6,8 +6,11 @@ brute force) of every row and drops entry [0] (the row itself); ``most_popular_n
 that occurs most often in the workload (first maximum; absent rows count 0).  The result per table is the alt-key array the
 C3 tier reads: ``alt_row * 100 + alt_table`` with tables numbered from 1 (convert_altkeys_to_binary.py:50).
 
-Here both steps are ``evs_knn`` (csrc/evs_knn.cuh): one fused tensor-core kernel (3xTF32 ``mma.sync`` distances, fp32
-accurate, with the top-11 selection in registers) and a merge kernel that also makes the popularity pick.
+Here both steps are ``evs_knn`` (csrc/evs_knn.cuh): one fused tensor-core kernel (3xTF32 ``mma.sync`` distances: every
+operand split into hi, rounded to TF32, and the exact remainder lo, which the tensor core truncates; fp32 accurate, with
+the top-11 selection in registers) and a merge kernel that also makes the popularity pick.  A row with a NaN or ±Inf
+element (or one whose squared norm overflows fp32) is never a neighbour or an alt key; such a row's own neighbours are
+all -1 and its alt key is 0.
 """
 from __future__ import annotations
 

@@ -9,9 +9,13 @@
 //
 // k_knn -- fused distance + selection.  A CTA owns 128 query rows and walks a range of the database in tiles of 64 rows:
 //   * dist(q, x) is ranked by |x|^2 - 2 q.x; the dot products of a 128 x 64 tile run on the tensor cores
-//     (mma.sync.m16n8k8 TF32, warp w = query rows 16w .. 16w+15).  Operands are split hi + lo (rounded to TF32's mantissa
-//     with integer adds) and a product is hi*hi + hi*lo + lo*hi, i.e. fp32-accurate: a neighbour list is only as good as
-//     its near-ties, and plain TF32 (10 mantissa bits) reorders them.  The split of a database tile is done ONCE, by the
+//     (mma.sync.m16n8k8 TF32, warp w = query rows 16w .. 16w+15).  Operands are split hi + lo (hi = the value rounded to
+//     TF32's mantissa with an integer add, lo = the exact remainder, which the tensor core truncates to TF32) and a product
+//     is hi*hi + hi*lo + lo*hi, within 5 * 2^-22 of the exact product: a neighbour list is only as good as its near-ties,
+//     and plain TF32 (10 mantissa bits) reorders them.  lo is not rounded: the rounding add carries a NaN's mantissa into
+//     the sign bit (0x7FFFFFFF -> -0.0), so a NaN row would rank as a zero row.  Unrounded, lo is NaN for a NaN or +-Inf
+//     element, every ranking value of its row (or query) is NaN and never passes a threshold: such a row is never a
+//     neighbour, such a query gets none.  The split of a database tile is done ONCE, by the
 //     thread that stages it (global -> registers -> hi / lo planes in shared memory, the next tile's loads in flight under
 //     the current tile's math); the queries' split fragments live in registers for d <= 16;
 //   * every thread keeps, for each of its two query rows, a sorted list (in shared memory) of the 11 best (distance, index)
@@ -83,7 +87,7 @@ __global__ void __launch_bounds__(kKnnThreads, 2) k_knn(const float *__restrict_
         if (q0 + r < nq && c < D) v = __ldg(q + (q0 + r) * D + c);
         const unsigned h = tf32_rn(v);
         s_qhi[r * ld + c] = h;
-        s_qlo[r * ld + c] = tf32_rn(v - __uint_as_float(h));
+        s_qlo[r * ld + c] = __float_as_uint(v - __uint_as_float(h));      // exact; NaN for NaN / Inf (see the header)
     }
     __syncthreads();
     // A fragments of this warp's 16 query rows; logical k slots tq / tq + 4 of a k-step take columns k0 + 2 tq, k0 + 2 tq + 1
@@ -143,7 +147,8 @@ __global__ void __launch_bounds__(kKnnThreads, 2) k_knn(const float *__restrict_
     };
     // |x|^2 of a tile's rows: when a row's pieces sit in d4 neighbouring lanes (d4 = 2, 4, 8, 16) the lanes add up their pieces
     // in a fixed butterfly (the same x gets the same norm in every CTA: the ranking must not depend on who computed it), else
-    // one thread per row walks the row in shared memory.  Rows past the end of the range get +inf: never selected.
+    // one thread per row walks the row in shared memory (hi + lo there is the value itself, or NaN for a NaN or Inf: the
+    // norm is never finite for a non-finite row on either path).  Rows past the end of the range get +inf: never selected.
     const bool shfl_norm = (32 % d4) == 0;
     auto store_tile = [&](long long base) {
         __syncthreads();                                     // the previous tile's reads are over
@@ -159,7 +164,7 @@ __global__ void __launch_bounds__(kKnnThreads, 2) k_knn(const float *__restrict_
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 hp[k] = tf32_rn(v[k]);
-                lp[k] = tf32_rn(v[k] - __uint_as_float(hp[k]));
+                lp[k] = __float_as_uint(v[k] - __uint_as_float(hp[k]));
                 nn = fmaf(v[k], v[k], nn);
             }
             if (on) {

@@ -312,7 +312,9 @@ int evs_store_ptr(evs_handle h, int tier, int table, const void **dev_ptr, int32
  * convert_altkeys_to_binary.py:50).  One fused tensor-core kernel (distances by 3xTF32 mma.sync: fp32-accurate) + a merge.
  *   x_dev  fp32 [n][dim] the database (n < 2^31, dim <= 64);  q_dev fp32 [nq][dim] the query rows (may point into x_dev)
  *   nbr_dev int64 [nq][k] global row ids, nearest first (ties by index), -1 where the database has fewer rows; or NULL
- *   dist_dev fp32 [nq][k] squared distances, or NULL
+ *   dist_dev fp32 [nq][k] squared distances (non-finite where nbr is -1), or NULL
+ *   A database row with a NaN or +-Inf element, or whose squared norm overflows fp32, is never a neighbour or an alt key;
+ *   a query row with a NaN or +-Inf element gets -1 everywhere, non-finite distances and alt key 0.
  *   alt_dev uint32 [nq] alt keys, or NULL; then table_off_dev int64 [n_tables + 1] = first global row of each table and
  *           freq_dev uint32 [n] request counts per global row (or NULL: every neighbour counts 0, the nearest wins) */
 int evs_knn(const float *x_dev, int64_t n, const float *q_dev, int64_t nq, int32_t dim, int32_t k, int64_t *nbr_dev,
