@@ -51,7 +51,7 @@ class EvsStats(C.Structure):
 
 # every symbol include/evstore_b200.h declares
 SYMBOLS = [
-    "evs_create", "evs_destroy", "evs_last_error", "evs_version", "evs_lookup_batch", "evs_lookup_batches", "evs_lookup_bags", "evs_note_replays", "evs_prefetch", "evs_update_rows", "evs_probe_batch", "evs_check",
+    "evs_create", "evs_destroy", "evs_last_error", "evs_version", "evs_lookup_batch", "evs_lookup_batches", "evs_lookup_bags", "evs_note_replays", "evs_prefetch", "evs_update_rows", "evs_state_bytes", "evs_save_state", "evs_load_state", "evs_probe_batch", "evs_check",
     "evs_memory_footprint", "evs_host_alloc", "evs_host_free",
     "evs_lookup_batch_host", "evs_submit_host", "evs_wait_host", "evs_sync", "evs_stats", "evs_last_events", "evs_dump_state", "evs_dump_c3",
     "evs_interact", "evs_knn", "evs_embedding_bag", "evs_embedding_bag_status", "evs_store_ptr", "evs_shard_create", "evs_shard_export",
@@ -92,6 +92,12 @@ def load_library(path: str | None = None):
     lib.evs_prefetch.restype = C.c_int
     lib.evs_update_rows.argtypes = [vp, vp, i64, vp, i64, vp, vp]
     lib.evs_update_rows.restype = C.c_int
+    lib.evs_state_bytes.argtypes = [vp, C.POINTER(C.c_uint64)]
+    lib.evs_state_bytes.restype = C.c_int
+    lib.evs_save_state.argtypes = [vp, vp, C.c_uint64, C.POINTER(C.c_uint64), vp]
+    lib.evs_save_state.restype = C.c_int
+    lib.evs_load_state.argtypes = [vp, vp, C.c_uint64, vp]
+    lib.evs_load_state.restype = C.c_int
     lib.evs_check.argtypes = [vp, C.c_int]
     lib.evs_check.restype = C.c_int
     lib.evs_memory_footprint.argtypes = [vp, C.POINTER(C.c_uint64)]

@@ -8,6 +8,7 @@ fallback: construction raises when the CUDA library or a CUDA device is missing.
 from __future__ import annotations
 
 import ctypes as C
+import struct
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -61,6 +62,56 @@ def _stream_handle(stream, device):
         return stream
     import torch
     return torch.cuda.current_stream(device).cuda_stream or CUDA_STREAM_LEGACY
+
+
+STATE_MAGIC = b"EVSSTATE"
+STATE_VERSION = 1
+STATE_HEADER = struct.Struct("<8sIIQ8i3Q32i32q")         # include/evstore_b200.h: the snapshot header, 464 bytes
+
+
+def state_info(blob) -> dict:
+    """Header and section sizes of a snapshot from ``EvStore.save_state`` (no GPU): policy, n_layers, n_tables_total,
+    table_ids, rows, dim, precisions, capacities, and per tier n_perfect and the keys per bucket, C3's size and window
+    length.  Raises ValueError for a truncated or foreign blob."""
+    b = memoryview(np.ascontiguousarray(np.frombuffer(blob, dtype=np.uint8) if isinstance(blob, (bytes, bytearray)) else blob,
+                                        dtype=np.uint8)).cast("B")
+    if len(b) < STATE_HEADER.size:
+        raise ValueError(f"not a snapshot: {len(b)} bytes, shorter than the {STATE_HEADER.size}-byte header")
+    f = STATE_HEADER.unpack_from(b, 0)
+    magic, version, hdr, total = f[0], f[1], f[2], f[3]
+    if magic != STATE_MAGIC:
+        raise ValueError("not a snapshot (bad magic)")
+    if version != STATE_VERSION or hdr != STATE_HEADER.size:
+        raise ValueError(f"unsupported snapshot version {version}")
+    if total != len(b):
+        raise ValueError(f"snapshot of {len(b)} bytes, its header says {total}")
+    policy, n_layers, t_total, n_tables, dim, mp, sp, nb = f[4:12]
+    caps, c3_cap = list(f[12:14]), f[14]
+    ids, rows = list(f[15:15 + 32])[:n_tables], list(f[47:47 + 32])[:n_tables]
+    if not 1 <= n_layers <= 3 or not 1 <= n_tables <= 32 or not 2 <= nb <= 32:
+        raise ValueError("snapshot header out of range")
+    w = np.frombuffer(b, dtype="<u8", offset=STATE_HEADER.size) if (len(b) - STATE_HEADER.size) % 8 == 0 else None
+    if w is None:
+        raise ValueError("the snapshot body is not a whole number of 8-byte words")
+    o, tiers = 0, []
+    for _ in range(2 if n_layers >= 2 else 1):
+        if o + 1 + nb > len(w):
+            raise ValueError("truncated snapshot")
+        counts = [int(x) for x in w[o + 1:o + 1 + nb]]
+        tiers.append({"n_perfect": int(w[o]), "counts": counts})
+        o += 1 + nb + sum(counts)
+    c3 = None
+    if n_layers == 3 and c3_cap > 0:
+        if o + 2 > len(w):
+            raise ValueError("truncated snapshot")
+        c3 = {"size": int(w[o]), "window": int(w[o + 1])}
+        o += 2 + c3["window"] + 2 * c3["size"]
+    if o != len(w):
+        raise ValueError(f"snapshot body of {len(w)} words, its sections need {o}")
+    return {"version": version, "bytes": total, "policy": ("evlfu", "lru", "lfu")[policy] if 0 <= policy <= 2 else policy,
+            "n_layers": n_layers, "n_tables_total": t_total, "table_ids": ids, "rows": rows, "dim": dim,
+            "main_precision": mp, "secondary_precision": sp, "capacity": caps[:len(tiers)], "c3_capacity": c3_cap,
+            "tiers": tiers, "c3": c3}
 
 
 class _DevArray:
@@ -241,6 +292,31 @@ class EvStore:
         rc = self.lib.evs_update_rows(self.handle, keys.data_ptr(), n, values.data_ptr(), vstride, where.data_ptr(), st)
         _native.check(rc, "evs_update_rows")
         return where
+
+    def save_state(self, stream=None) -> np.ndarray:
+        """Snapshot of the cache's policy state (evs_save_state): resident keys per tier in eviction order, n_perfect,
+        C3's raw FIFO window and map -- keys only, no row bytes.  Reflects every lookup enqueued on ``stream`` (default:
+        torch's current stream) before the call; synchronises.  Returns the blob as a uint8 array (``state_info``
+        parses its header); ``load_state`` restores it into a handle serving the same tables."""
+        import torch
+        st = _stream_handle(stream, torch.device("cuda", self.cfg.device))
+        bound = C.c_uint64(0)
+        _native.check(self.lib.evs_state_bytes(self.handle, C.byref(bound)), "evs_state_bytes")
+        buf = np.empty(int(bound.value), dtype=np.uint8)
+        n = C.c_uint64(0)
+        _native.check(self.lib.evs_save_state(self.handle, buf.ctypes.data, buf.nbytes, C.byref(n), st), "evs_save_state")
+        return buf[:n.value].copy()
+
+    def load_state(self, blob, stream=None):
+        """Replace the cache's policy state with a snapshot from ``save_state`` (evs_load_state); rows are read from this
+        store's backing rows at its own precisions.  Lookups enqueued on ``stream`` after the call see the loaded state;
+        synchronises.  Raises EvsError for a snapshot of another configuration (the cache is then unchanged) or one whose
+        keys fail the device checks (the cache is then empty)."""
+        import torch
+        st = _stream_handle(stream, torch.device("cuda", self.cfg.device))
+        b = np.ascontiguousarray(np.frombuffer(blob, dtype=np.uint8) if isinstance(blob, (bytes, bytearray)) else blob,
+                                 dtype=np.uint8)
+        _native.check(self.lib.evs_load_state(self.handle, b.ctypes.data, b.nbytes, st), "evs_load_state")
 
     def check(self, clear: bool = False):
         """Raise if a batch that has already run saw an out-of-range index or a silent peer (no synchronisation)."""

@@ -19,6 +19,7 @@
 #include "evs_bags.cuh"
 #include "evs_knn.cuh"
 #include "evs_refresh.cuh"
+#include "evs_state.cuh"
 
 namespace evs {
 
@@ -322,6 +323,7 @@ static void free_all(evs_handle h) {
     if (h->upd_key) cudaFree(h->upd_key);
     if (h->upd_pos) cudaFree(h->upd_pos);
     if (h->ev_upd) cudaEventDestroy(h->ev_upd);
+    if (h->state_buf) cudaFree(h->state_buf);
     release_host_ranges(h);
     h->prof.destroy();
     if (h->pf_stream) cudaStreamDestroy(h->pf_stream);
@@ -1502,50 +1504,323 @@ int evs_last_events(evs_handle h, int tier, int64_t *evicted, int64_t *n_evicted
     return EVS_OK;
 }
 
+// ---- snapshots of the policy state (evs_state.cuh) ---------------------------------------------------------------
+// Blob = StateHeader, then per tier: n_perfect, count[n_buckets], the keys bucket by bucket (FIFO order); then, with three
+// layers: C3's size, the window length W, the W records, and size map entries (key, alt | flag << 32).  u64 words, little
+// endian (include/evstore_b200.h).
+struct StateHeader {
+    char magic[8];                           // "EVSSTATE"
+    uint32_t version, header_bytes;
+    uint64_t total_bytes;
+    int32_t policy, n_layers, n_tables_total, n_tables;
+    int32_t dim, main_precision, secondary_precision, n_buckets;   // precisions and capacities: informational
+    uint64_t cap[EVS_MAX_TIERS], c3_cap;
+    int32_t table_ids[EVS_MAX_TABLES];       // unused entries -1
+    int64_t rows[EVS_MAX_TABLES];            // unused entries 0
+};
+static_assert(sizeof(StateHeader) == 464 && sizeof(StateHeader) % 8 == 0, "snapshot header layout");
+static const char kStateMagic[8] = {'E', 'V', 'S', 'S', 'T', 'A', 'T', 'E'};
+constexpr uint32_t kStateVersion = 1;
+
+// Upper bound of the body's words: every tier full, C3 full with a full ring window.
+static unsigned long long state_body_bound(evs_handle h) {
+    unsigned long long w = 0;
+    for (int t = 0; t < h->n_tiers; ++t) w += 1ull + h->tier[t].dev.n_buckets + h->tier[t].dev.cap;
+    if (h->c3_active) w += 2ull + h->params.c3.ring_cap + 2ull * h->params.c3.cap;
+    return w;
+}
+
+static int state_reserve(evs_handle h, unsigned long long body_words) {
+    const size_t need = kStateMetaWords + body_words;
+    if (need <= h->state_words) return EVS_OK;
+    EVS_CUDA(cudaDeviceSynchronize());                        // an earlier call's kernels may still use the buffer
+    if (h->state_buf) cudaFree(h->state_buf);
+    h->hbm_bytes -= h->state_words * sizeof(unsigned long long);
+    h->state_buf = nullptr;
+    h->state_words = 0;
+    EVS_CUDA(cudaMalloc(&h->state_buf, need * sizeof(unsigned long long)));
+    h->state_words = need;
+    h->hbm_bytes += need * sizeof(unsigned long long);
+    return EVS_OK;
+}
+
+static bool state_capturing(cudaStream_t st) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    return cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone;
+}
+
+// k_state_save on st, then a synchronise: meta[0] = body words, meta[1] = status, meta[2 + 32 t + b] = live records.
+static int state_stage(evs_handle h, cudaStream_t st, unsigned long long (&meta)[kStateMetaWords], const char *what) {
+    int rc = state_reserve(h, state_body_bound(h));
+    if (rc) return rc;
+    EVS_CUDA(cudaMemsetAsync(h->state_buf, 0, kStateMetaWords * sizeof(unsigned long long), st));
+    {
+        LaunchScope ls(h->prof, K_STATE, st);
+        const int ctas = h->n_tiers * h->tier[0].dev.n_buckets + (h->c3_active ? 1 : 0);
+        k_state_save<<<ctas, kStateThreads, 0, st>>>(h->params, h->state_buf);
+        EVS_CUDA(cudaGetLastError());
+    }
+    EVS_CUDA(cudaMemcpyAsync(meta, h->state_buf, sizeof(meta), cudaMemcpyDeviceToHost, st));
+    EVS_CUDA(cudaStreamSynchronize(st));
+    if (meta[1] & kStateOverCap) {
+        set_error(std::string(what) + ": a tier holds more keys than its capacity");
+        return EVS_ERR_CAPACITY;
+    }
+    return EVS_OK;
+}
+
+static int state_c3_ok(const unsigned long long (&meta)[kStateMetaWords], const char *what) {
+    if (!(meta[1] & kStateBadC3)) return EVS_OK;
+    set_error(std::string(what) + ": C3's map entries differ from its size");
+    return EVS_ERR_CAPACITY;
+}
+
+// The body words of tier `tier` (n_perfect, count[], keys) within the staged body.
+static size_t state_tier_offset(evs_handle h, const std::vector<unsigned long long> &body, int tier) {
+    size_t o = 0;
+    for (int t = 0; t < tier; ++t) {
+        const int nb = h->tier[t].dev.n_buckets;
+        unsigned long long n = 0;
+        for (int b = 0; b < nb; ++b) n += body[o + 1 + b];
+        o += 1 + nb + n;
+    }
+    return o;
+}
+
+static int state_fetch_body(evs_handle h, cudaStream_t st, const unsigned long long (&meta)[kStateMetaWords], void *dst) {
+    if (meta[0]) EVS_CUDA(cudaMemcpyAsync(dst, h->state_buf + kStateMetaWords, meta[0] * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    EVS_CUDA(cudaStreamSynchronize(st));
+    return EVS_OK;
+}
+
+int evs_state_bytes(evs_handle h, uint64_t *bound) {
+    if (h == nullptr || bound == nullptr) return EVS_ERR_INVALID;
+    *bound = sizeof(StateHeader) + state_body_bound(h) * sizeof(unsigned long long);
+    return EVS_OK;
+}
+
+int evs_save_state(evs_handle h, void *buf, uint64_t cap, uint64_t *bytes, void *stream) {
+    if (h == nullptr || buf == nullptr || bytes == nullptr) {
+        set_error("evs_save_state: bad handle / pointers");
+        return EVS_ERR_INVALID;
+    }
+    DeviceGuard dg(h->cfg.device);
+    cudaStream_t st = stream_of(h, stream);
+    if (state_capturing(st)) {
+        set_error("evs_save_state: the stream is being captured; call it outside a graph, between launches");
+        return EVS_ERR_INVALID;
+    }
+    unsigned long long meta[kStateMetaWords];
+    int rc = state_stage(h, st, meta, "evs_save_state");
+    if (rc) return rc;
+    if (meta[1] & kStateBadBucket) {
+        set_error("evs_save_state: a bucket's live records differ from its count");
+        return EVS_ERR_CAPACITY;
+    }
+    if ((rc = state_c3_ok(meta, "evs_save_state"))) return rc;
+    const uint64_t total = sizeof(StateHeader) + meta[0] * sizeof(unsigned long long);
+    *bytes = total;
+    if (cap < total) {
+        set_error("evs_save_state: buffer of " + std::to_string(cap) + " B, the snapshot needs " + std::to_string(total) + " B");
+        return EVS_ERR_INVALID;
+    }
+    StateHeader hd{};
+    memcpy(hd.magic, kStateMagic, 8);
+    hd.version = kStateVersion;
+    hd.header_bytes = sizeof(StateHeader);
+    hd.total_bytes = total;
+    hd.policy = h->cfg.policy;
+    hd.n_layers = h->cfg.n_layers;
+    hd.n_tables_total = h->cfg.n_tables_total;
+    hd.n_tables = h->cfg.n_tables;
+    hd.dim = h->cfg.dim;
+    hd.main_precision = h->tier[0].prec;
+    hd.secondary_precision = h->n_tiers == 2 ? h->tier[1].prec : 0;
+    hd.n_buckets = h->tier[0].dev.n_buckets;
+    for (int t = 0; t < h->n_tiers; ++t) hd.cap[t] = h->tier[t].dev.cap;
+    hd.c3_cap = h->c3_active ? h->params.c3.cap : 0;
+    for (int t = 0; t < EVS_MAX_TABLES; ++t) {
+        hd.table_ids[t] = t < h->cfg.n_tables ? h->table_ids[t] : -1;
+        hd.rows[t] = t < h->cfg.n_tables ? h->rows[t] : 0;
+    }
+    memcpy(buf, &hd, sizeof(hd));
+    return state_fetch_body(h, st, meta, static_cast<unsigned char *>(buf) + sizeof(StateHeader));
+}
+
+// Parses and checks a snapshot against the handle on the host; fills the load arguments (offsets into the body).
+static int state_parse(evs_handle h, const unsigned char *buf, uint64_t bytes, StateLoadArgs &a, size_t &body_words,
+                       size_t &win_off, size_t &map_off) {
+    auto bad = [](const std::string &m) {
+        set_error("evs_load_state: " + m);
+        return EVS_ERR_INVALID;
+    };
+    if (bytes < sizeof(StateHeader)) return bad("truncated: " + std::to_string(bytes) + " B is shorter than the header");
+    StateHeader hd;
+    memcpy(&hd, buf, sizeof(hd));
+    if (memcmp(hd.magic, kStateMagic, 8) != 0) return bad("not a snapshot (bad magic)");
+    if (hd.version != kStateVersion || hd.header_bytes != sizeof(StateHeader))
+        return bad("unsupported snapshot version " + std::to_string(hd.version));
+    if (hd.total_bytes != bytes) return bad("length " + std::to_string(bytes) + " B, the header says " + std::to_string(hd.total_bytes) + " B");
+    if ((bytes - sizeof(StateHeader)) % 8 != 0) return bad("the body is not a whole number of 8-byte words");
+    if (hd.policy != h->cfg.policy) return bad("policy " + std::to_string(hd.policy) + " != " + std::to_string(h->cfg.policy));
+    if (hd.n_layers != h->cfg.n_layers) return bad("n_layers " + std::to_string(hd.n_layers) + " != " + std::to_string(h->cfg.n_layers));
+    if (hd.n_tables_total != h->cfg.n_tables_total) return bad("n_tables_total differs");
+    if (hd.n_tables != h->cfg.n_tables || hd.n_buckets != h->tier[0].dev.n_buckets) return bad("the served tables differ");
+    for (int t = 0; t < h->cfg.n_tables; ++t) {
+        if (hd.table_ids[t] != h->table_ids[t]) return bad("the served tables differ");
+        if (hd.rows[t] != h->rows[t]) return bad("rows of table " + std::to_string(h->table_ids[t]) + " differ");
+    }
+    const unsigned long long *w = reinterpret_cast<const unsigned long long *>(buf + sizeof(StateHeader));
+    const size_t nw = (bytes - sizeof(StateHeader)) / 8;
+    size_t o = 0;
+    const int nb = h->tier[0].dev.n_buckets;
+    a = StateLoadArgs{};
+    for (int t = 0; t < h->n_tiers; ++t) {
+        if (o + 1 + nb > nw) return bad("truncated in tier " + std::to_string(t));
+        if (w[o] > 0xFFFFFFFFull) return bad("n_perfect out of range");
+        a.n_perfect[t] = static_cast<unsigned>(w[o]);
+        unsigned long long n = 0;
+        a.off[t][0] = 0;
+        for (int b = 0; b < nb; ++b) {
+            n += w[o + 1 + b];
+            if (n > h->tier[t].dev.cap)
+                return bad("tier " + std::to_string(t) + " holds more keys than this handle's capacity " + std::to_string(h->tier[t].dev.cap));
+            a.off[t][b + 1] = static_cast<unsigned>(n);
+        }
+        o += 1 + nb;
+        if (o + n > nw) return bad("truncated in tier " + std::to_string(t));
+        a.keys[t] = reinterpret_cast<const unsigned long long *>(o * 8);      // offset; the device address is added later
+        o += n;
+    }
+    win_off = map_off = 0;
+    if (h->c3_active) {
+        if (o + 2 > nw) return bad("truncated in C3");
+        const unsigned long long size = w[o], W = w[o + 1];
+        const unsigned long long c3cap = h->params.c3.cap, ring = h->params.c3.ring_cap;
+        if (size > c3cap) return bad("C3 holds " + std::to_string(size) + " keys, more than this handle's capacity " + std::to_string(c3cap));
+        // the next batch's c3_update appends up to the victims of both tiers behind the window (evs_c3.cuh)
+        const unsigned long long room = 2ull * static_cast<unsigned long long>(h->cfg.max_batch) * h->cfg.n_tables;
+        if (W + room > ring)
+            return bad("C3's window of " + std::to_string(W) + " records leaves no room for a batch's " + std::to_string(room) +
+                       " appends in this handle's ring of " + std::to_string(ring));
+        o += 2;
+        if (o + W + 2 * size > nw) return bad("truncated in C3");
+        win_off = o;
+        a.W = W;
+        o += W;
+        map_off = o;
+        a.n_map = static_cast<unsigned>(size);
+        o += 2 * size;
+    }
+    if (o != nw) return bad("the body has " + std::to_string(nw) + " words, its sections " + std::to_string(o));
+    body_words = nw;
+    return EVS_OK;
+}
+
+// Clears every tier and C3 and, with a = the parsed snapshot, loads it (k_init_* -> k_state_load[_c3] -> k_state_load_ctl).
+static int state_install(evs_handle h, cudaStream_t st, const StateLoadArgs &a, bool load) {
+    LaunchScope ls(h->prof, K_STATE, st);
+    for (int t = 0; t < h->n_tiers; ++t) k_init_tier<<<592, 256, 0, st>>>(h->tier[t].dev);
+    if (h->c3_active) k_init_c3<<<592, 256, 0, st>>>(h->params.c3);
+    EVS_CUDA(cudaGetLastError());
+    // no programmatic serialization: the next batch's k_serve cannot start before the state is complete
+    void *args[] = {&h->params, const_cast<StateLoadArgs *>(&a)};
+    if (load) {
+        const unsigned n = a.off[0][h->tier[0].dev.n_buckets] + (h->n_tiers == 2 ? a.off[1][h->tier[1].dev.n_buckets] : 0u);
+        if (n) EVS_CUDA(launch_ex(reinterpret_cast<const void *>(k_state_load), dim3(std::min<unsigned>((n + 7) / 8, 148 * 16)), 256, 0, st, args, false));
+        if (h->c3_active && a.n_map + a.W)
+            EVS_CUDA(launch_ex(reinterpret_cast<const void *>(k_state_load_c3), dim3(static_cast<unsigned>(std::min<unsigned long long>((a.n_map + a.W + 255) / 256, 148 * 8))),
+                               256, 0, st, args, false));
+    }
+    EVS_CUDA(launch_ex(reinterpret_cast<const void *>(k_state_load_ctl), dim3(1), 32, 0, st, args, false));
+    return EVS_OK;
+}
+
+int evs_load_state(evs_handle h, const void *buf, uint64_t bytes, void *stream) {
+    if (h == nullptr || buf == nullptr) {
+        set_error("evs_load_state: bad handle / pointer");
+        return EVS_ERR_INVALID;
+    }
+    DeviceGuard dg(h->cfg.device);
+    cudaStream_t st = stream_of(h, stream);
+    if (state_capturing(st)) {
+        set_error("evs_load_state: the stream is being captured; call it outside a graph, between launches");
+        return EVS_ERR_INVALID;
+    }
+    StateLoadArgs a;
+    size_t body_words = 0, win_off = 0, map_off = 0;
+    int rc = state_parse(h, static_cast<const unsigned char *>(buf), bytes, a, body_words, win_off, map_off);
+    if (rc) return rc;
+    if ((rc = state_reserve(h, body_words))) return rc;
+    if (h->ev_upd == nullptr) EVS_CUDA(cudaEventCreateWithFlags(&h->ev_upd, cudaEventDisableTiming));
+    unsigned long long *body = h->state_buf + kStateMetaWords;
+    EVS_CUDA(cudaMemsetAsync(h->state_buf, 0, kStateMetaWords * sizeof(unsigned long long), st));
+    if (body_words)
+        EVS_CUDA(cudaMemcpyAsync(body, static_cast<const unsigned char *>(buf) + sizeof(StateHeader), body_words * 8, cudaMemcpyHostToDevice, st));
+    for (int t = 0; t < h->n_tiers; ++t) a.keys[t] = body + reinterpret_cast<uintptr_t>(a.keys[t]) / 8;
+    a.window = body + win_off;
+    a.map = body + map_off;
+    a.err = reinterpret_cast<unsigned *>(h->state_buf + 1);
+    if ((rc = state_install(h, st, a, true))) return rc;
+    // the look-ahead: an announcement made before the load staged rows of the old state's misses -- cancel it, and order
+    // every later k_prefetch behind the new state (as evs_update_rows does)
+    h->pf.cancel();
+    EVS_CUDA(cudaEventRecord(h->ev_upd, st));
+    EVS_CUDA(cudaStreamWaitEvent(h->pf_stream, h->ev_upd, 0));
+    unsigned long long err = 0;
+    EVS_CUDA(cudaMemcpyAsync(&err, h->state_buf + 1, sizeof(err), cudaMemcpyDeviceToHost, st));
+    EVS_CUDA(cudaStreamSynchronize(st));
+    if (err) {
+        StateLoadArgs empty{};
+        if ((rc = state_install(h, st, empty, false))) return rc;
+        EVS_CUDA(cudaStreamSynchronize(st));
+    }
+    // the ring-occupancy mirror (maintain_rings): the device is idle, the rings hold count records from position 0
+    for (int t = 0; t < h->n_tiers; ++t) {
+        unsigned long long mx = 0;
+        if (!err)
+            for (int b = 0; b < h->tier[t].dev.n_buckets; ++b) mx = std::max<unsigned long long>(mx, a.off[t][b + 1] - a.off[t][b]);
+        *reinterpret_cast<volatile unsigned long long *>(h->ring_host + t) = (static_cast<unsigned long long>(static_cast<unsigned>(h->seq)) << 32) | mx;
+    }
+    if (err) {
+        set_error(std::string("evs_load_state: ") + ((err & kStateBadKey) ? "a key's table is not served here or its row is out of range"
+                                                                            : "a key appears twice in one tier or in C3's map") +
+                  "; the handle is now empty");
+        return EVS_ERR_INVALID;
+    }
+    return EVS_OK;
+}
+
 int evs_dump_state(evs_handle h, int tier, int64_t *keys, int64_t *n_keys, int64_t *bucket_off, int64_t *n_perfect) {
     if (h == nullptr || tier < 0 || tier >= h->n_tiers || keys == nullptr || n_keys == nullptr || bucket_off == nullptr)
         return EVS_ERR_INVALID;
     EVS_CUDA(cudaSetDevice(h->cfg.device));
     EVS_CUDA(cudaDeviceSynchronize());
-    const TierDev &d = h->tier[tier].dev;
-    TierCtl c;
-    EVS_CUDA(cudaMemcpy(&c, d.ctl, sizeof(c), cudaMemcpyDeviceToHost));
-    std::vector<Slot> slots(static_cast<size_t>(d.hash_mask) + 1);
-    EVS_CUDA(cudaMemcpy(slots.data(), d.slots, sizeof(Slot) * slots.size(), cudaMemcpyDeviceToHost));
+    unsigned long long meta[kStateMetaWords];
+    int rc = state_stage(h, h->stream, meta, "evs_dump_state");
+    if (rc) return rc;
+    std::vector<unsigned long long> body(meta[0]);
+    if ((rc = state_fetch_body(h, h->stream, meta, body.data()))) return rc;
+    const int nb = h->tier[tier].dev.n_buckets;
+    const size_t o = state_tier_offset(h, body, tier);
     int64_t n = 0;
-    std::vector<unsigned> rec;
-    for (int b = 0; b < d.n_buckets; ++b) {
-        bucket_off[b] = n;
-        const unsigned long long len = c.tail[b] - c.head[b];
-        rec.resize(len);
-        for (unsigned long long done = 0; done < len;) {        // the live window may wrap the ring
-            const unsigned long long pos = (c.head[b] + done) & (d.ring_cap - 1);
-            const unsigned long long run = std::min<unsigned long long>(len - done, d.ring_cap - pos);
-            EVS_CUDA(cudaMemcpy(rec.data() + done, d.ring + static_cast<size_t>(b) * d.ring_cap + pos, sizeof(unsigned) * run,
-                                cudaMemcpyDeviceToHost));
-            done += run;
-        }
-        unsigned live = 0;
-        for (unsigned long long i = 0; i < len; ++i) {
-            const unsigned sl = rec[i];
-            if (sl <= d.hash_mask && slots[sl].meta == pack_meta(b, c.head[b] + i)) {
-                if (n >= *n_keys) {
-                    set_error("evs_dump_state: keys array too small");
-                    return EVS_ERR_INVALID;
-                }
-                keys[n++] = static_cast<int64_t>(slots[sl].kw & kKeyMask);
-                ++live;
-            }
-        }
-        if (live != c.count[b]) {
-            set_error("evs_dump_state: bucket " + std::to_string(b) + " live records " + std::to_string(live) +
-                      " != count " + std::to_string(c.count[b]));
+    for (int b = 0; b < nb; ++b) {
+        const unsigned long long cnt = body[o + 1 + b], live = meta[2 + kMaxBuckets * tier + b];
+        if (live != cnt) {
+            set_error("evs_dump_state: bucket " + std::to_string(b) + " live records " + std::to_string(live) + " != count " + std::to_string(cnt));
             return EVS_ERR_CAPACITY;
         }
+        bucket_off[b] = n;
+        if (n + static_cast<int64_t>(cnt) > *n_keys) {
+            set_error("evs_dump_state: keys array too small");
+            return EVS_ERR_INVALID;
+        }
+        for (unsigned long long i = 0; i < cnt; ++i) keys[n + i] = static_cast<int64_t>(body[o + 1 + nb + n + i]);
+        n += static_cast<int64_t>(cnt);
     }
-    bucket_off[d.n_buckets] = n;
+    bucket_off[nb] = n;
     *n_keys = n;
-    if (n_perfect) *n_perfect = c.n_perfect;
+    if (n_perfect) *n_perfect = static_cast<int64_t>(body[o]);
     return EVS_OK;
 }
 
@@ -1559,35 +1834,27 @@ int evs_dump_c3(evs_handle h, int64_t *keys, uint32_t *alt, uint8_t *recency, in
     }
     EVS_CUDA(cudaSetDevice(h->cfg.device));
     EVS_CUDA(cudaDeviceSynchronize());
-    const C3Dev &d = h->params.c3;
-    C3Ctl c;
-    EVS_CUDA(cudaMemcpy(&c, d.ctl, sizeof(c), cudaMemcpyDeviceToHost));
-    std::vector<C3Slot> slots(static_cast<size_t>(d.hash_mask) + 1);
-    EVS_CUDA(cudaMemcpy(slots.data(), d.slots, sizeof(C3Slot) * slots.size(), cudaMemcpyDeviceToHost));
-    std::vector<unsigned long long> ring(d.ring_cap);
-    EVS_CUDA(cudaMemcpy(ring.data(), d.ring, sizeof(unsigned long long) * d.ring_cap, cudaMemcpyDeviceToHost));
+    unsigned long long meta[kStateMetaWords];
+    int rc = state_stage(h, h->stream, meta, "evs_dump_c3");
+    if (rc || (rc = state_c3_ok(meta, "evs_dump_c3"))) return rc;
+    std::vector<unsigned long long> body(meta[0]);
+    if ((rc = state_fetch_body(h, h->stream, meta, body.data()))) return rc;
+    const size_t o = state_tier_offset(h, body, h->n_tiers);
+    const unsigned long long size = body[o], W = body[o + 1];
+    const unsigned long long *win = body.data() + o + 2, *map = win + W;
+    std::map<unsigned long long, unsigned long long> mapped;
+    for (unsigned long long i = 0; i < size; ++i) mapped[map[2 * i]] = map[2 * i + 1];
     int64_t cnt = 0;
-    for (unsigned long long q = c.head; q < c.tail; ++q) {
-        const unsigned long long key = ring[q & (d.ring_cap - 1)];
-        unsigned i = hash_key(key, d.hash_mask);
-        bool found = false;
-        while (true) {
-            const unsigned long long kw = slots[i].kw;
-            if ((kw & kKeyMask) == key) {
-                found = true;
-                break;
-            }
-            if ((kw >> 48) == 0ull) break;
-            i = (i + 1) & d.hash_mask;
-        }
-        if (!found) continue;
+    for (unsigned long long q = 0; q < W; ++q) {
+        const auto it = mapped.find(win[q]);
+        if (it == mapped.end()) continue;
         if (cnt >= *n) {
             set_error("evs_dump_c3: arrays too small");
             return EVS_ERR_INVALID;
         }
-        if (keys) keys[cnt] = static_cast<int64_t>(key);
-        if (alt) alt[cnt] = slots[i].alt;
-        if (recency) recency[cnt] = static_cast<uint8_t>(slots[i].flag & 1u);
+        if (keys) keys[cnt] = static_cast<int64_t>(win[q]);
+        if (alt) alt[cnt] = static_cast<uint32_t>(it->second);
+        if (recency) recency[cnt] = static_cast<uint8_t>((it->second >> 32) & 1u);
         ++cnt;
     }
     *n = cnt;

@@ -38,9 +38,9 @@ struct Tier {
 
 
 // Kernel ids for the launch counter / per-kernel CUDA-event timing (evs_set_profiling).
-enum KernelId { K_SERVE = 0, K_SCAN, K_UPDATE, K_EVICT, K_PREFETCH, K_COMPACT, K_PROBE, K_INTERACT, K_GATHER, K_BAGS, K_UPDATE_ROWS, K_COUNT };
+enum KernelId { K_SERVE = 0, K_SCAN, K_UPDATE, K_EVICT, K_PREFETCH, K_COMPACT, K_PROBE, K_INTERACT, K_GATHER, K_BAGS, K_UPDATE_ROWS, K_STATE, K_COUNT };
 static const char *const kKernelNames[K_COUNT] = {"k_serve", "k_scan", "k_update", "k_evict", "k_prefetch", "k_compact", "k_probe", "k_interact",
-                                                  "k_gather", "k_bags", "k_update_rows"};
+                                                  "k_gather", "k_bags", "k_update_rows", "k_state"};
 
 struct Profiler {
     bool on = false;
@@ -153,7 +153,10 @@ struct evs_handle_s {
     unsigned long long *upd_key = nullptr;
     long long *upd_pos = nullptr;
     size_t upd_cap = 0;                      // entries of each (a power of two, >= 2 n)
-    cudaEvent_t ev_upd = nullptr;            // after the last update: orders the look-ahead stream behind it
+    cudaEvent_t ev_upd = nullptr;            // after the last update or state load: orders the look-ahead stream behind it
+    // evs_save_state / evs_load_state / evs_dump_*: staging of a snapshot's body behind kStateMetaWords words (grown, synchronously)
+    unsigned long long *state_buf = nullptr;
+    size_t state_words = 0;
     // staging for the host-buffer paths: slot 0 serves the synchronous call, all kPipeSlots the
     // pipelined one (H2D of batch n+1 and D2H of batch n-1 overlap the kernels of batch n)
     static constexpr int kPipeSlots = 4;

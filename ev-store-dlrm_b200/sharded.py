@@ -192,6 +192,14 @@ class ShardedLookup:
             where[sel] = self.store.update_rows(t, rows[sel], values[sel], stream=stream)
         return where
 
+    def save_state(self):
+        """Snapshot of this rank's cache (``EvStore.save_state``)."""
+        return self.store.save_state()
+
+    def load_state(self, blob):
+        """Restore a snapshot of a rank that served the same tables (``EvStore.load_state``); re-sharding is not supported."""
+        self.store.load_state(blob)
+
     def alltoall_bytes(self, B: int) -> int:
         """Bytes this rank sends to its peers per batch (SURVEY.md section 8(d))."""
         return B * self.T_local * self.dim * 4 * (self.world - 1) // self.world

@@ -16,6 +16,7 @@
  *                                                                      one batch, a queue of batches, bags with pooling)
  *        evs_prefetch, evs_note_replays                                look-ahead; the lookup inside a caller's CUDA graph
  *        evs_update_rows                                               new row values, ordered between batches
+ *        evs_state_bytes / evs_save_state / evs_load_state             snapshot of a warm cache's policy state, and restore
  *        evs_shard_*                                                   table-wise sharding over NVLink peer memory
  *        evs_embedding_bag, evs_interact, evs_knn                      the ops either side of the cache; alt-key generation
  *        evs_host_alloc / evs_host_free                                host memory for backing rows (large device pages)
@@ -200,6 +201,42 @@ int evs_prefetch(evs_handle h, const int64_t *idx_dev, int32_t B, void *ready_ev
  * allowed while `stream` is being captured (EVS_ERR_INVALID).  n == 0 is a no-op. */
 int evs_update_rows(evs_handle h, const int64_t *keys_dev, int64_t n, const float *values_dev, int64_t value_stride,
                     uint8_t *where_dev, void *stream);
+
+/* ---- snapshots of the policy state: keep a warm cache across a restart ------------------------------- *
+ * A snapshot holds a handle's policy state with KEYS ONLY: per tier (C1, C2) its resident keys bucket by bucket in
+ * eviction (FIFO) order and n_perfect; for C3 the raw FIFO window, stale and duplicate records included, and the map
+ * entries (key, alt key, recency flag).  Rows are re-read from the loading handle's backing store at its own
+ * precisions, so a snapshot survives evs_update_rows and loads into a handle whose tiers use other precisions.
+ * Guarantee: handle A saves after some batches, handle B loads the snapshot; given the same batches from then on, A and
+ * B return bit-identical rows, hit codes and agg_hit, the same evs_last_events streams, evs_dump_state / evs_dump_c3
+ * and statistics deltas, for every policy and lookup path.  Slot assignments may differ; nothing observable depends
+ * on them.  Loading replaces the whole state (B may have served traffic).
+ * The loading handle must match policy, n_layers, n_tables_total, the served global table ids and rows[]; each tier's
+ * key count and C3's size must fit its capacities, and C3's window must leave room in its ring for one batch's
+ * appends (2 * max_batch * n_tables records).  dim, precisions, max_batch, larger
+ * capacities, store_in_hbm and the device may differ.
+ *
+ * Blob, little-endian: a 464-byte header
+ *     char magic[8] "EVSSTATE"; u32 version (1); u32 header bytes (464); u64 total bytes;
+ *     i32 policy, n_layers, n_tables_total, n_tables; i32 dim, main_precision, secondary_precision, n_buckets;
+ *     u64 cap[2], c3_cap; i32 table_ids[32] (-1 past n_tables); i64 rows[32] (0 past n_tables)
+ *     (dim, precisions and capacities are informational), then u64 words:
+ *     per tier (1 or 2):  n_perfect; count[n_buckets]; the keys, (global table << 40) | row, bucket 0 first, each
+ *                         bucket oldest first
+ *     C3 (three layers):  size; W; the W window records, oldest first; size map entries (key, alt | flag << 32)
+ *
+ * evs_state_bytes: an upper bound of a snapshot's size, from the capacities (no synchronisation).
+ * evs_save_state: writes the snapshot into buf (host memory of any kind, cap bytes) and its size into *bytes
+ *   (EVS_ERR_INVALID with *bytes set when cap is too small).  Reflects every batch enqueued on `stream` before it.
+ * evs_load_state: replaces the handle's state with the snapshot; every batch enqueued on `stream` after it sees it.
+ *   It cancels a pending evs_prefetch announcement and leaves the cumulative statistics alone.  The header and
+ *   every count are checked on the host first: a mismatch returns EVS_ERR_INVALID with the reason in evs_last_error and
+ *   the handle untouched.  The device then checks each key (table served, row in range, at most once per tier, C3 map
+ *   keys unique); a key that fails returns EVS_ERR_INVALID and leaves the handle EMPTY, as after evs_create.
+ * Both are stream-ordered, synchronise before returning, and are refused while `stream` is being captured. */
+int evs_state_bytes(evs_handle h, uint64_t *bound);
+int evs_save_state(evs_handle h, void *buf, uint64_t cap, uint64_t *bytes, void *stream);
+int evs_load_state(evs_handle h, const void *buf, uint64_t bytes, void *stream);
 
 /* Probe only: per-sample local hit counts (for the sharded exact mode the ranks
  * all-reduce these and pass the sum back as agg_in).  Does not change state. */
