@@ -51,11 +51,11 @@ class EvsStats(C.Structure):
 
 # every symbol include/evstore_b200.h declares
 SYMBOLS = [
-    "evs_create", "evs_destroy", "evs_last_error", "evs_version", "evs_lookup_batch", "evs_lookup_batches", "evs_lookup_bags", "evs_note_replays", "evs_prefetch", "evs_update_rows", "evs_state_bytes", "evs_save_state", "evs_load_state", "evs_probe_batch", "evs_check",
+    "evs_create", "evs_destroy", "evs_last_error", "evs_version", "evs_lookup_batch", "evs_lookup_batches", "evs_lookup_bags", "evs_lookup_bags_agg", "evs_probe_bags", "evs_note_replays", "evs_prefetch", "evs_update_rows", "evs_state_bytes", "evs_save_state", "evs_load_state", "evs_probe_batch", "evs_check",
     "evs_memory_footprint", "evs_host_alloc", "evs_host_free",
     "evs_lookup_batch_host", "evs_submit_host", "evs_wait_host", "evs_sync", "evs_stats", "evs_last_events", "evs_dump_state", "evs_dump_c3",
     "evs_interact", "evs_knn", "evs_embedding_bag", "evs_embedding_bag_status", "evs_store_ptr", "evs_shard_create", "evs_shard_export",
-    "evs_shard_connect", "evs_shard_lookup", "evs_shard_lookup_many", "evs_shard_destroy", "evs_set_profiling", "evs_kernel_times", "evs_launch_count", "evs_phase_times", "evs_legacy_configure", "evs_legacy_handle", "ev_lookup", "get_ev_values", "print_perfect_hit",
+    "evs_shard_connect", "evs_shard_lookup", "evs_shard_lookup_many", "evs_shard_lookup_bags", "evs_shard_destroy", "evs_set_profiling", "evs_kernel_times", "evs_launch_count", "evs_phase_times", "evs_legacy_configure", "evs_legacy_handle", "ev_lookup", "get_ev_values", "print_perfect_hit",
     "test_arr", "ev_lookup_based_on_list_keys",
 ]
 
@@ -86,6 +86,10 @@ def load_library(path: str | None = None):
     lib.evs_lookup_batches.restype = C.c_int
     lib.evs_lookup_bags.argtypes = [vp, vp, vp, i32, i64, i32, vp, i64, vp, vp]
     lib.evs_lookup_bags.restype = C.c_int
+    lib.evs_lookup_bags_agg.argtypes = [vp, vp, vp, i32, i64, i32, vp, i64, vp, vp, vp]
+    lib.evs_lookup_bags_agg.restype = C.c_int
+    lib.evs_probe_bags.argtypes = [vp, vp, vp, i32, i64, i32, vp, vp]
+    lib.evs_probe_bags.restype = C.c_int
     lib.evs_note_replays.argtypes = [vp, i64, vp]
     lib.evs_note_replays.restype = C.c_int
     lib.evs_prefetch.argtypes = [vp, vp, i32, vp]
@@ -144,6 +148,8 @@ def load_library(path: str | None = None):
     lib.evs_shard_lookup.restype = C.c_int
     lib.evs_shard_lookup_many.argtypes = [vp, i32, vp, i32, vp, vp, vp]
     lib.evs_shard_lookup_many.restype = C.c_int
+    lib.evs_shard_lookup_bags.argtypes = [vp, vp, vp, i32, i64, i32, vp, C.POINTER(vp), vp]
+    lib.evs_shard_lookup_bags.restype = C.c_int
     lib.evs_shard_destroy.argtypes = [vp]
     lib.evs_shard_destroy.restype = C.c_int
     lib.evs_set_profiling.argtypes = [vp, C.c_int]

@@ -351,10 +351,8 @@ class EvStore:
         st = _stream_handle(stream, torch.device("cuda", self.cfg.device))
         _native.check(self.lib.evs_note_replays(self.handle, int(n), st), "evs_note_replays")
 
-    def lookup_bags(self, lS_o, lS_i, max_per_bag: int = 10, out=None, stream=None):
-        """Pooled lookup (evs_lookup_bags): lS_i / lS_o are the per-table index and offset tensors of apply_emb
-        (lS_i[t] int64 CUDA [nnz_t], lS_o[t] int64 CUDA [B], nn.EmbeddingBag's offsets).  Returns (pooled fp32
-        [B, n_tables, dim], hit: list of n_tables uint8 tensors [nnz_t])."""
+    def _pack_bags(self, lS_o, lS_i):
+        """apply_emb's per-table lists -> (B, nnz per table, idx int64 [nnz] table 0 first, off int64 [n_tables*B + 1])."""
         import torch
         T = self.n_tables
         assert len(lS_i) == T and len(lS_o) == T
@@ -365,14 +363,42 @@ class EvStore:
         idx = torch.cat([x.reshape(-1).to(torch.int64) for x in lS_i]) if base[-1] > 0 else torch.zeros(1, dtype=torch.int64, device=dev)
         off = torch.cat([lS_o[t].reshape(-1).to(torch.int64) + int(base[t]) for t in range(T)] +
                         [torch.tensor([int(base[-1])], dtype=torch.int64, device=dev)])
+        return B, base, idx, off
+
+    def lookup_bags(self, lS_o, lS_i, max_per_bag: int = 10, out=None, stream=None, agg_in=None):
+        """Pooled lookup (evs_lookup_bags): lS_i / lS_o are the per-table index and offset tensors of apply_emb
+        (lS_i[t] int64 CUDA [nnz_t], lS_o[t] int64 CUDA [B], nn.EmbeddingBag's offsets).  Returns (pooled fp32
+        [B, n_tables, dim], hit: list of n_tables uint8 tensors [nnz_t]).  agg_in: uint8 CUDA [B * max_per_bag], each
+        slice's agg_hit summed over the ranks of a sharded cache (evs_lookup_bags_agg, after ``probe_bags``), or None."""
+        import torch
+        T = self.n_tables
+        B, base, idx, off = self._pack_bags(lS_o, lS_i)
+        dev = idx.device
         if out is None:
             out = torch.empty((B, T, self.dim), dtype=torch.float32, device=dev)
         hit = torch.empty((max(int(base[-1]), 1),), dtype=torch.uint8, device=dev)
         st = _stream_handle(stream, dev)
-        rc = self.lib.evs_lookup_bags(self.handle, idx.data_ptr(), off.data_ptr(), B, int(base[-1]), int(max_per_bag),
-                                      out.data_ptr(), out.stride(0), hit.data_ptr(), st)
-        _native.check(rc, "evs_lookup_bags")
+        if agg_in is None:
+            rc = self.lib.evs_lookup_bags(self.handle, idx.data_ptr(), off.data_ptr(), B, int(base[-1]), int(max_per_bag),
+                                          out.data_ptr(), out.stride(0), hit.data_ptr(), st)
+            _native.check(rc, "evs_lookup_bags")
+        else:
+            assert agg_in.is_cuda and agg_in.dtype == torch.uint8 and agg_in.numel() >= B * int(max_per_bag)
+            rc = self.lib.evs_lookup_bags_agg(self.handle, idx.data_ptr(), off.data_ptr(), B, int(base[-1]), int(max_per_bag),
+                                              out.data_ptr(), out.stride(0), hit.data_ptr(), agg_in.data_ptr(), st)
+            _native.check(rc, "evs_lookup_bags_agg")
         return out, [hit[int(base[t]):int(base[t + 1])] for t in range(T)]
+
+    def probe_bags(self, lS_o, lS_i, max_per_bag: int = 10, agg_out=None, stream=None):
+        """Local hit count of every slice of a bag batch (evs_probe_bags): uint8 [B * max_per_bag].  State is unchanged."""
+        import torch
+        B, base, idx, off = self._pack_bags(lS_o, lS_i)
+        if agg_out is None:
+            agg_out = torch.empty((max(B * int(max_per_bag), 1),), dtype=torch.uint8, device=idx.device)
+        st = _stream_handle(stream, idx.device)
+        _native.check(self.lib.evs_probe_bags(self.handle, idx.data_ptr(), off.data_ptr(), B, int(base[-1]), int(max_per_bag),
+                                              agg_out.data_ptr(), st), "evs_probe_bags")
+        return agg_out
 
     def lookup_many(self, lS_i_list, outs=None, hits=None, stream=None):
         """Consecutive batches in one call (evs_lookup_batches): the same results as ``lookup`` on each in turn, but groups
@@ -528,6 +554,21 @@ class EvStore:
         _native.check(self.lib.evs_shard_lookup_many(self._shard, n, ip, B, hp, op, st), "evs_shard_lookup_many")
         shape = (B // self._shard_world, self.cfg.n_tables_total or self.n_tables, self.dim)
         return [_tensor_from_ptr(op[i], shape, dev) for i in range(n)], hits
+
+    def shard_lookup_bags(self, lS_o, lS_i, max_per_bag: int = 10, stream=None):
+        """Bags on a rank of a sharded cache (evs_shard_lookup_bags): lS_o / lS_i as ``lookup_bags`` for this rank's tables
+        over the whole global batch.  Returns (this rank's pooled [B/world, n_tables_total, dim] rows, valid until four
+        batches later; hit: list of n_tables uint8 tensors [nnz_t])."""
+        import torch
+        B, base, idx, off = self._pack_bags(lS_o, lS_i)
+        dev = idx.device
+        hit = torch.empty((max(int(base[-1]), 1),), dtype=torch.uint8, device=dev)
+        st = _stream_handle(stream, dev)
+        ptr = C.c_void_p()
+        _native.check(self.lib.evs_shard_lookup_bags(self._shard, idx.data_ptr(), off.data_ptr(), B, int(base[-1]), int(max_per_bag),
+                                                     hit.data_ptr(), C.byref(ptr), st), "evs_shard_lookup_bags")
+        shape = (B // self._shard_world, self.cfg.n_tables_total or self.n_tables, self.dim)
+        return _tensor_from_ptr(ptr.value, shape, dev), [hit[int(base[t]):int(base[t + 1])] for t in range(self.n_tables)]
 
     def shard_destroy(self):
         if getattr(self, "_shard", None):

@@ -1119,61 +1119,130 @@ int evs_lookup_batches(evs_handle h, int32_t n, const int64_t *const *idx_dev, i
 }
 
 // Bags (pooling factor > 1) on the cached path: see evs_bags.cuh.
-int evs_lookup_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
-                    float *out_dev, int64_t out_stride, uint8_t *hit_dev, void *stream) {
+static int bags_check(evs_handle h, const char *what, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz,
+                      int32_t max_per_bag, long long max_slices) {
     if (h == nullptr || B < 0 || nnz < 0 || max_per_bag < 1 || max_per_bag > kMaxPerBag || off_dev == nullptr ||
-        (B > 0 && out_dev == nullptr) || (nnz > 0 && idx_dev == nullptr)) {
-        set_error("evs_lookup_bags: bad handle / B / nnz / max_per_bag (1..32) / pointers");
+        (nnz > 0 && idx_dev == nullptr)) {
+        set_error(std::string(what) + ": bad handle / B / nnz / max_per_bag (1..32) / pointers");
         return EVS_ERR_INVALID;
     }
-    if (static_cast<long long>(B) * max_per_bag > h->cfg.max_batch) {
-        set_error("evs_lookup_bags: B * max_per_bag slices exceed max_batch (create the handle with max_batch >= B * max_per_bag)");
+    if (static_cast<long long>(B) * max_per_bag > max_slices) {
+        set_error(std::string(what) + ": B * max_per_bag slices exceed the largest batch (max_batch, or batch_max of evs_shard_create)");
         return EVS_ERR_INVALID;
     }
-    if (h->sharded) {
-        set_error("evs_lookup_bags: not available on a rank of a table-wise sharded cache");
-        return EVS_ERR_INVALID;
-    }
-    if (B == 0) return EVS_OK;
-    DeviceGuard dg(h->cfg.device);
-    cudaStream_t st = stream_of(h, stream);
-    const int T = h->cfg.n_tables, D = h->cfg.dim, P = max_per_bag;
-    if (h->bag_idx == nullptr) {                              // slice scratch, on first use
+    return EVS_OK;
+}
+
+// The batch's slices: scratch on first use (slice rows W tables wide: a table's rows sit at its output column p.col[t],
+// which is its global id once the handle is a rank of a sharded cache), then k_bags_expand.
+static int bags_expand(evs_handle h, cudaStream_t st, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int P) {
+    const int T = h->cfg.n_tables, D = h->cfg.dim;
+    const int W = h->sharded ? h->cfg.n_tables_total : T;
+    if (h->bag_idx == nullptr || h->bag_cols < W) {
         t_alloc_bytes = &h->hbm_bytes;
         struct AllocScope {
             ~AllocScope() { t_alloc_bytes = nullptr; }
         } alloc_scope;
         const long long n_max = static_cast<long long>(h->cfg.max_batch) * T;
         int rc;
-        if ((rc = dev_alloc(h->dev_allocs, &h->bag_idx, n_max))) return rc;
-        if ((rc = dev_alloc(h->dev_allocs, &h->bag_rows, n_max * D))) return rc;
-        if ((rc = dev_alloc(h->dev_allocs, &h->bag_hit, n_max))) return rc;
+        if (h->bag_idx == nullptr) {
+            if ((rc = dev_alloc(h->dev_allocs, &h->bag_idx, n_max))) return rc;
+            if ((rc = dev_alloc(h->dev_allocs, &h->bag_hit, n_max))) return rc;
+        } else {                                              // bags before evs_shard_connect: the rows grow to W tables
+            EVS_CUDA(cudaDeviceSynchronize());
+            h->dev_allocs.erase(std::find(h->dev_allocs.begin(), h->dev_allocs.end(), static_cast<void *>(h->bag_rows)));
+            EVS_CUDA(cudaFree(h->bag_rows));
+            h->hbm_bytes -= static_cast<size_t>(h->cfg.max_batch) * h->bag_cols * D * sizeof(float);
+        }
+        if ((rc = dev_alloc(h->dev_allocs, &h->bag_rows, static_cast<long long>(h->cfg.max_batch) * W * D))) return rc;
+        h->bag_cols = W;
     }
-    const int Bv = B * P;
-    const long long total = static_cast<long long>(Bv) * T;
-    {
-        LaunchScope ls(h->prof, K_BAGS, st);
-        k_bags_expand<<<static_cast<unsigned>(std::min<long long>((total + 255) / 256, 148 * 8)), 256, 0, st>>>(
-            h->params, reinterpret_cast<const long long *>(idx_dev), reinterpret_cast<const long long *>(off_dev), B, P, nnz, h->bag_idx);
-        EVS_CUDA(cudaGetLastError());
-    }
-    BatchArgs a = lookup_args(h, reinterpret_cast<const int64_t *>(h->bag_idx), Bv, h->bag_rows, 0, h->bag_hit);
-    a.bags = 1;
-    int rc = submit_batch(h, st, a);
-    if (rc) return rc;
-    {
-        LaunchScope ls(h->prof, K_BAGS, st);
-        const long long os = out_stride > 0 ? out_stride : static_cast<long long>(T) * D;
-        const bool vec = (D & 3) == 0 && (os & 3) == 0 && (reinterpret_cast<uintptr_t>(out_dev) & 15u) == 0;
-        const long long items = static_cast<long long>(B) * T * (vec ? D / 4 : D);
-        const unsigned grid = static_cast<unsigned>(std::min<long long>((items + 255) / 256, 148 * 16));
-        if (vec)
-            k_bags_pool<true><<<grid, 256, 0, st>>>(h->bag_rows, h->bag_hit, reinterpret_cast<const long long *>(off_dev), B, P, T, D, out_dev, os, hit_dev);
-        else
-            k_bags_pool<false><<<grid, 256, 0, st>>>(h->bag_rows, h->bag_hit, reinterpret_cast<const long long *>(off_dev), B, P, T, D, out_dev, os, hit_dev);
-        EVS_CUDA(cudaGetLastError());
-    }
+    const long long total = static_cast<long long>(B) * P * T;
+    LaunchScope ls(h->prof, K_BAGS, st);
+    k_bags_expand<<<static_cast<unsigned>(std::min<long long>((total + 255) / 256, 148 * 8)), 256, 0, st>>>(
+        h->params, reinterpret_cast<const long long *>(idx_dev), reinterpret_cast<const long long *>(off_dev), B, P, nnz, h->bag_idx);
+    EVS_CUDA(cudaGetLastError());
     return EVS_OK;
+}
+
+// The arguments of the slice batch bags_expand staged: B*P slices, rows into the slice staging.
+static BatchArgs bags_args(evs_handle h, int32_t B, int P) {
+    BatchArgs a = lookup_args(h, reinterpret_cast<const int64_t *>(h->bag_idx), B * P, h->bag_rows,
+                              static_cast<long long>(h->bag_cols) * h->cfg.dim, h->bag_hit);
+    a.bags = 1;
+    return a;
+}
+
+// k_bags_pool over the staged slice rows: into out (one GPU) or, sh.world > 1, into the owner ranks' receive buffers.
+static int bags_pool(evs_handle h, cudaStream_t st, const ShardArgs &sh, const int64_t *off_dev, int32_t B, int P, int64_t nnz, float *out_dev,
+                     int64_t out_stride, uint8_t *hit_dev) {
+    LaunchScope ls(h->prof, K_BAGS, st);
+    const int T = h->cfg.n_tables, D = h->cfg.dim;
+    const long long os = out_stride > 0 ? out_stride : static_cast<long long>(T) * D;
+    const bool vec = (D & 3) == 0 && (sh.world > 1 || ((os & 3) == 0 && (reinterpret_cast<uintptr_t>(out_dev) & 15u) == 0));
+    const long long items = static_cast<long long>(B) * T * (vec ? D / 4 : D);
+    const unsigned grid = static_cast<unsigned>(std::min<long long>((items + 255) / 256, 148 * 16));
+    const long long *off = reinterpret_cast<const long long *>(off_dev);
+    if (vec)
+        k_bags_pool<true><<<grid, 256, 0, st>>>(h->params, sh, h->bag_rows, h->bag_hit, off, B, P, nnz, h->bag_cols, out_dev, os, hit_dev);
+    else
+        k_bags_pool<false><<<grid, 256, 0, st>>>(h->params, sh, h->bag_rows, h->bag_hit, off, B, P, nnz, h->bag_cols, out_dev, os, hit_dev);
+    EVS_CUDA(cudaGetLastError());
+    return EVS_OK;
+}
+
+static int lookup_bags(evs_handle h, const char *what, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz,
+                       int32_t max_per_bag, float *out_dev, int64_t out_stride, uint8_t *hit_dev, const uint8_t *agg_in, void *stream) {
+    int rc = bags_check(h, what, idx_dev, off_dev, B, nnz, max_per_bag, h ? h->cfg.max_batch : 0);
+    if (rc) return rc;
+    if (B > 0 && out_dev == nullptr) {
+        set_error(std::string(what) + ": null output");
+        return EVS_ERR_INVALID;
+    }
+    if (h->sharded) {
+        set_error(std::string(what) + ": not available on a rank of a table-wise sharded cache (evs_shard_lookup_bags is)");
+        return EVS_ERR_INVALID;
+    }
+    if (B == 0) return EVS_OK;
+    DeviceGuard dg(h->cfg.device);
+    cudaStream_t st = stream_of(h, stream);
+    const int P = max_per_bag;
+    if ((rc = bags_expand(h, st, idx_dev, off_dev, B, nnz, P))) return rc;
+    BatchArgs a = bags_args(h, B, P);
+    a.agg_in = agg_in;
+    if ((rc = submit_batch(h, st, a))) return rc;
+    return bags_pool(h, st, ShardArgs{}, off_dev, B, P, nnz, out_dev, out_stride, hit_dev);
+}
+
+int evs_lookup_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                    float *out_dev, int64_t out_stride, uint8_t *hit_dev, void *stream) {
+    return lookup_bags(h, "evs_lookup_bags", idx_dev, off_dev, B, nnz, max_per_bag, out_dev, out_stride, hit_dev, nullptr, stream);
+}
+
+int evs_lookup_bags_agg(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                        float *out_dev, int64_t out_stride, uint8_t *hit_dev, const uint8_t *agg_in, void *stream) {
+    if (agg_in == nullptr && B > 0) {
+        set_error("evs_lookup_bags_agg: null agg_in");
+        return EVS_ERR_INVALID;
+    }
+    return lookup_bags(h, "evs_lookup_bags_agg", idx_dev, off_dev, B, nnz, max_per_bag, out_dev, out_stride, hit_dev, agg_in, stream);
+}
+
+int evs_probe_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                   uint8_t *agg_out_dev, void *stream) {
+    int rc = bags_check(h, "evs_probe_bags", idx_dev, off_dev, B, nnz, max_per_bag, h ? h->cfg.max_batch : 0);
+    if (rc) return rc;
+    if (B > 0 && agg_out_dev == nullptr) {
+        set_error("evs_probe_bags: null agg_out");
+        return EVS_ERR_INVALID;
+    }
+    if (B == 0) return EVS_OK;
+    DeviceGuard dg(h->cfg.device);
+    cudaStream_t st = stream_of(h, stream);
+    if ((rc = bags_expand(h, st, idx_dev, off_dev, B, nnz, max_per_bag))) return rc;
+    BatchArgs a = bags_args(h, B, max_per_bag);
+    a.agg_out = agg_out_dev;
+    return launch_probe(h, a, st);
 }
 
 // New values for the rows of n keys (evs_refresh.cuh), stream-ordered between batches.
@@ -2056,6 +2125,37 @@ int evs_shard_lookup_many(evs_shard s, int32_t n, const int64_t *const *idx_dev,
     if (rc) return rc;
     DeviceGuard dg(s->h->cfg.device);
     return shard_submit(s, stream_of(s->h, stream), n, idx_dev, B, hit_dev, out_dev);
+}
+
+// Bags on a rank of a sharded cache: the rank's tables' bags of the whole global batch as B*P slices whose agg_hit counts
+// go through the exchange (fused or a separate probe pass, as for a plain batch); the slice rows stay in the handle's
+// staging, and k_bags_pool sends the pooled rows to the owner ranks and closes the epoch.  One batch per call: no
+// grouping, no look-ahead.  Plain and bags batches share the epoch sequence and the four receive buffers.
+int evs_shard_lookup_bags(evs_shard s, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                          uint8_t *hit_dev, float **out_dev, void *stream) {
+    if (s == nullptr || out_dev == nullptr) {
+        set_error("evs_shard_lookup_bags: null pointer");
+        return EVS_ERR_INVALID;
+    }
+    int rc = bags_check(s->h, "evs_shard_lookup_bags", idx_dev, off_dev, B, nnz, max_per_bag, s->batch_max);
+    if (rc || (rc = shard_check(s, "evs_shard_lookup_bags", B))) return rc;
+    evs_handle h = s->h;
+    DeviceGuard dg(h->cfg.device);
+    cudaStream_t st = stream_of(h, stream);
+    const int P = max_per_bag;
+    if ((rc = bags_expand(h, st, idx_dev, off_dev, B, nnz, P))) return rc;
+    const unsigned epoch = s->epoch + 1;
+    const int64_t *slices = reinterpret_cast<const int64_t *>(h->bag_idx);
+    rc = submit_batches(h, st, 1, &slices, B * P, false, [&](int, BatchArgs &a) {
+        s->epoch = epoch;
+        a = bags_args(h, B, P);
+        a.sh = shard_args(s, B * P, epoch);                  // the count tables are indexed by slice
+        return s->fused ? EVS_OK : launch_probe(h, a, st);
+    });
+    if (rc) return rc;
+    if ((rc = bags_pool(h, st, shard_args(s, B, epoch), off_dev, B, P, nnz, nullptr, 0, hit_dev))) return rc;   // by pooled sample
+    *out_dev = reinterpret_cast<float *>(s->block + s->off_recv + (epoch % evs_shard_s::kRecvBufs) * s->recv_bytes);
+    return EVS_OK;
 }
 
 int evs_shard_destroy(evs_shard s) {

@@ -145,10 +145,12 @@ struct evs_handle_s {
     evs::BatchArgs *d_args = nullptr;        // device copy of the per-batch arguments
     long long *d_rows = nullptr;
     uint8_t *d_agg = nullptr;                // [max_batch]
-    // evs_lookup_bags: the batch's slices (allocated on first use): indices [T][B*P], rows [B*P][T][D], hit codes [B*P][T]
+    // evs_lookup_bags / evs_shard_lookup_bags: the batch's slices (allocated on first use): indices [T][B*P],
+    // rows [B*P][bag_cols][D] (bag_cols = T, or n_tables_total on a rank of a sharded cache), hit codes [B*P][T]
     long long *bag_idx = nullptr;
     float *bag_rows = nullptr;
     uint8_t *bag_hit = nullptr;
+    int bag_cols = 0;
     // evs_update_rows: scratch hash of one call's keys (grown, synchronously, when a call brings more keys)
     unsigned long long *upd_key = nullptr;
     long long *upd_pos = nullptr;

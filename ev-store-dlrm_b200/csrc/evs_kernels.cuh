@@ -48,13 +48,15 @@ __device__ __forceinline__ void griddep_launch(const Params &p) {
 
 // Where the fp32 rows of sample s go: the caller's buffer, or -- table-wise sharded -- the receive
 // buffer of the rank that owns the sample (peer memory over NVLink).  Local table t lands at column p.col[t].
+// A bags batch keeps its slice rows local on a sharded handle too (a.out: the handle's slice staging); k_bags_pool sends
+// the pooled rows.
 __device__ __forceinline__ float *out_row(const BatchArgs &a, const Params &p, int s) {
-    if (a.sh.world <= 1) return a.out + static_cast<size_t>(s) * a.out_stride;
+    if (a.sh.world <= 1 || a.bags) return a.out + static_cast<size_t>(s) * a.out_stride;
     const int dst = s / a.sh.Bl, ls = s - dst * a.sh.Bl;
     return a.sh.recv[dst] + static_cast<size_t>(ls) * a.sh.T_total * p.D;
 }
 __device__ __forceinline__ bool out_vec_ok(const BatchArgs &a, int D) {
-    if (a.sh.world > 1) return (D & 3) == 0;              // receive buffers are cudaMalloc'ed blocks
+    if (a.sh.world > 1 && !a.bags) return (D & 3) == 0;   // receive buffers are cudaMalloc'ed blocks
     return ((reinterpret_cast<uintptr_t>(a.out) & 15u) == 0) && ((a.out_stride & 3) == 0) && ((D & 3) == 0);
 }
 __device__ __forceinline__ void set_error(const Params &p, unsigned code) {
@@ -223,7 +225,7 @@ __device__ __forceinline__ bool fetch_list_body(const Params &p, unsigned cta, u
     const int B = ga->B;
     float *out = ga->out;
     const long long out_stride = ga->out_stride;
-    const int world = ga->sh.world, Bl = ga->sh.Bl, T_total = ga->sh.T_total;
+    const int world = ga->bags ? 0 : ga->sh.world, Bl = ga->sh.Bl, T_total = ga->sh.T_total;   // bags: as out_row()
     const unsigned want_tag = ga->pf_gen << 1;
     const bool use_pf = ga->pf_gen != 0u;
     const unsigned par = ga->seq & 1u;

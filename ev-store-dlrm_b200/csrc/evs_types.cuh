@@ -139,6 +139,7 @@ struct GlobalCtl {
     unsigned int fetch_done_seq;           // number of the last batch whose miss-fetch role has finished (it no longer reads its staging rows)
     unsigned int auto_seq;                 // number of the last batch started; a batch launched with BatchArgs::seq == 0 (a replay of a
                                            // graph the CALLER captured: its arguments are frozen) takes the next number from here
+    unsigned int pool_arrived;             // k_bags_pool on a sharded handle: CTAs done with their pooled rows (the last resets it)
 };
 constexpr unsigned long long kPeerTimeoutNs = 4000000000ull;   // spin-waits on peer flags give up after 4 s
 
@@ -179,7 +180,9 @@ struct BatchArgs {
     int probe_only;
     unsigned seq;                          // number of this batch on the handle (>= 1)
     unsigned pf_gen;                       // != 0: evs_prefetch staged rows for this batch (Params::pf_*), tagged with this generation
-    int bags;                              // 1: the batch holds slices of ragged bags; a negative index = no key at that position
+    int bags;                              // 1: the batch holds slices of ragged bags; a negative index = no key at that position.
+                                           // Sharded: the counts still go through the exchange, but the slice rows stay local (out)
+                                           // and k_bags_pool sends the pooled rows and raises the completion words
     ShardArgs sh;
 };
 

@@ -422,7 +422,8 @@ __device__ __forceinline__ void close_batch(const Params &p) {
     unsigned long long used = 0ull;          // warp t < n_tiers: max over tier t's buckets of tail - head
     unsigned long long d = 0ull, t5 = 0ull;  // warp kPhaseWarp: p.dbg[lane], the closing CTA's start
     const unsigned seq = p.args->seq;
-    const int world = p.args->sh.world;
+    // a bags batch has delivered no rows yet: k_bags_pool raises and waits for the completion words after pooling
+    const int world = p.args->bags ? 0 : p.args->sh.world;
     if (warp < p.n_tiers) {
         const int t = warp, b = lane;
         const TierDev &tier = p.tier[t];

@@ -78,8 +78,8 @@ def split_cache_budget(rows_per_rank, total_rows_cached: int, floor: int = 1024)
 
 class ShardedLookup:
     """One rank's part of the sharded lookup.  ``store`` serves this rank's tables
-    (``EvStore`` built with table_base / n_tables_total; any object with ``probe`` and ``lookup``
-    of the same signatures works, which is how the CPU tests drive the host logic)."""
+    (``EvStore`` built with table_base / n_tables_total; any object with ``probe`` and ``lookup`` -- and ``probe_bags`` /
+    ``lookup_bags`` for bags -- of the same signatures works, which is how the CPU tests drive the host logic)."""
 
     def __init__(self, store, n_tables_total: int, dim: int, rank: int, world: int, group=None, exact_agg: bool = True,
                  transport: str = "nccl", batch_max: int = 0, placement=None):
@@ -123,7 +123,6 @@ class ShardedLookup:
         """lS_i_local: int64 [T_local, B], this rank's tables for the whole batch (B % world == 0).
         next_idx: the tensor the NEXT call will pass (look-ahead, EvStore.prefetch), or None.
         Returns (ly [B/world, 26, dim] for this rank's slice of the batch, hit [B, T_local])."""
-        import torch
         import torch.distributed as dist
         T_local, B = lS_i_local.shape
         assert T_local == self.T_local and B % self.world == 0
@@ -143,6 +142,34 @@ class ShardedLookup:
             self.store.prefetch(next_idx)
         if self.world == 1:
             return send, hit
+        return self._exchange(send, recv, out, B), hit
+
+    def lookup_bags(self, lS_o_local, lS_i_local, max_per_bag: int = 10):
+        """Bags (pooling factor > 1) of this rank's tables for the whole batch: lS_o_local / lS_i_local are apply_emb's
+        per-table offset and index tensors of this rank's T_local tables (B bags each, B % world == 0, bags of at most
+        max_per_bag indices).  A batch of bags is looked up as B * max_per_bag slices whose agg_hit is summed over the
+        ranks; each rank pools its own tables and only pooled rows cross between the ranks.
+        Returns (ly [B/world, 26, dim] for this rank's slice of the batch, hit: per local table uint8 [nnz_t])."""
+        import torch.distributed as dist
+        assert len(lS_o_local) == self.T_local and len(lS_i_local) == self.T_local
+        B = int(lS_o_local[0].numel())
+        assert B % self.world == 0
+        if self.transport == "p2p":
+            return self.store.shard_lookup_bags(lS_o_local, lS_i_local, max_per_bag)
+        send, recv, out, _, _ = self._buffers(B, lS_i_local[0].device)
+        agg_in = None
+        if self.exact_agg and self.world > 1:
+            agg_in = self.store.probe_bags(lS_o_local, lS_i_local, max_per_bag)
+            dist.all_reduce(agg_in, op=dist.ReduceOp.SUM, group=self.group)
+        _, hit = self.store.lookup_bags(lS_o_local, lS_i_local, max_per_bag, out=send, agg_in=agg_in)
+        if self.world == 1:
+            return send, hit
+        return self._exchange(send, recv, out, B), hit
+
+    def _exchange(self, send, recv, out, B):
+        """Table-sharded pooled rows [B, T_local, d] -> this rank's batch-sharded [B/world, 26, d] (all_to_all_single)."""
+        import torch
+        import torch.distributed as dist
         Bl = B // self.world
         # send: [B, T_local*d] split along the batch; recv: world blocks [Bl, T_src, d], source-rank major
         in_splits = [Bl * self.T_local * self.dim] * self.world
@@ -158,7 +185,7 @@ class ShardedLookup:
             else:
                 out[:, torch.as_tensor(ids, device=out.device), :] = blk
             o += n
-        return out, hit
+        return out
 
     def lookup_many(self, idx_list, next_idx=None, hits=None):
         """Consecutive batches in one call: [(ly, hit)] as ``lookup`` on each in turn.  With the fused transport groups of 4

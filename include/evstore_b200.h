@@ -14,6 +14,7 @@
  *        evs_create / evs_destroy / evs_stats / evs_check ...          handle life cycle and bookkeeping
  *        evs_lookup_batch / _batches / _bags / _batch_host / evs_submit_host   the hot path (device or host buffers,
  *                                                                      one batch, a queue of batches, bags with pooling)
+ *        evs_probe_batch / evs_probe_bags / evs_lookup_bags_agg        exact agg_hit over a collective transport
  *        evs_prefetch, evs_note_replays                                look-ahead; the lookup inside a caller's CUDA graph
  *        evs_update_rows                                               new row values, ordered between batches
  *        evs_state_bytes / evs_save_state / evs_load_state             snapshot of a warm cache's policy state, and restore
@@ -156,6 +157,15 @@ int evs_lookup_batch(evs_handle h, const int64_t *idx_dev, int32_t B, float *out
  * a request group in the reference's sense (its agg_hit counts the hits among its own keys). */
 int evs_lookup_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
                     float *out_dev, int64_t out_stride, uint8_t *hit_dev, void *stream);
+/* Bags for a table-wise sharded cache over a collective transport (probe -> all-reduce of the slice counts -> lookup ->
+ * all-to-all of the POOLED rows), the bags form of evs_probe_batch / evs_lookup_batch(agg_in):
+ *   evs_probe_bags      agg_out_dev uint8 [B*P]: each slice's local hit count (absent positions count nothing); no state change
+ *   evs_lookup_bags_agg agg_in uint8 [B*P]: each slice's agg_hit summed over the ranks; otherwise evs_lookup_bags
+ * Same arguments, limits and refusals as evs_lookup_bags (P = max_per_bag). */
+int evs_probe_bags(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                   uint8_t *agg_out_dev, void *stream);
+int evs_lookup_bags_agg(evs_handle h, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                        float *out_dev, int64_t out_stride, uint8_t *hit_dev, const uint8_t *agg_in, void *stream);
 
 /* n consecutive batches of B samples in one call: exactly the results of n evs_lookup_batch calls in that order (the
  * batches stay strictly ordered on the device), but groups of 4 batches go to the device as ONE captured graph, so only
@@ -325,6 +335,18 @@ int evs_shard_lookup(evs_shard s, const int64_t *idx_dev, int32_t B, uint8_t *hi
  * batch i; the buffers rotate through 4, so each stays valid until four batches later. */
 int evs_shard_lookup_many(evs_shard s, int32_t n, const int64_t *const *idx_dev, int32_t B, uint8_t *const *hit_dev,
                           float **out_dev, void *stream);
+/* Bags on a rank of a sharded cache: a sharded bag batch gives exactly what evs_lookup_bags gives on one GPU with every
+ * table, agg_hit summed over the ranks.  idx_dev / off_dev: the evs_lookup_bags layout for THIS rank's tables over the
+ * whole global batch B (a multiple of world).  Every rank expands its bags into B*P slices (slice s*P+j = the j-th index
+ * of each bag of sample s; P = max_per_bag <= 32, B*P <= batch_max); a slice's agg_hit is the sum over the ranks of the hits
+ * among its present keys, and each rank runs the policy on its slices.  The rank pools its tables locally (j ascending,
+ * single fp32 adds from +0.0; an empty bag gives zeros) and stores only the pooled rows into the owner ranks' receive
+ * buffers: *out_dev receives this rank's [B/world][n_tables_total][dim] buffer, each table at the column of its global
+ * id, valid until four batches later.  hit_dev uint8 [nnz] per index as evs_lookup_bags, or NULL.  Malformed offsets or a
+ * bag larger than P raise the sticky EVS_ERR_INDEX.  One batch per call (no grouping, no look-ahead); plain and bag
+ * batches share the epoch sequence and the receive buffers and may be mixed freely.  Every rank makes the same calls. */
+int evs_shard_lookup_bags(evs_shard s, const int64_t *idx_dev, const int64_t *off_dev, int32_t B, int64_t nnz, int32_t max_per_bag,
+                          uint8_t *hit_dev, float **out_dev, void *stream);
 int evs_shard_destroy(evs_shard s);
 
 /* ---- sum pooling: nn.EmbeddingBag(mode="sum") of apply_emb_ori_dlrm ------------------- *
